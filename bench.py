@@ -9,7 +9,13 @@ likelihood kernel over that batch.  `value` = evals/s with inputs resident in
 HBM (CUDA-event timed), `e2e` = the same batch through the host-buffer C-ABI
 call (H2D of the parameters and D2H of lnL inside the timed region).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+`--steps` sets the number of timed launches of each likelihood path (device-resident, host-buffer pinned and
+pageable, Gaussian model).  `--dump-outputs DIR` writes the lnL arrays the device-resident NH3 and Gaussian
+calls returned in their last timed step as DIR/nh3_lnl.npy and DIR/gauss_lnl.npy (float64, 8 MB per GPU each,
+all ranks in rank order; a fixed seeded sample beyond 64 MB in all, see `dump_outputs`); the inputs are seeded,
+so two builds run with the same arguments can be compared output for output.
 
 `--impl reference` times the reference's own CPU implementation of the same path
 (oracle/_ref = the unmodified reference compiled by oracle/build_ref.py; the C
@@ -278,7 +284,7 @@ def run_ours(args):
 
     for _ in range(2):
         e2e_call()
-    n_e2e = max(3, min(args.steps, 10))
+    n_e2e = args.steps
     barrier()
     t0 = time.perf_counter()
     for _ in range(n_e2e):
@@ -306,10 +312,15 @@ def run_ours(args):
         dist.all_reduce(times, op=dist.ReduceOp.MAX)
     total_ms, e2e_s, e2e_pg_s = float(times[0]), float(times[1]), float(times[2])
 
-    gauss_result = run_gauss(nb, lib, _lib, dev, rank, dist) if not args.no_gauss else None
+    outputs = {"nh3_lnl": d_lnl}
+    gauss_result = None
+    if not args.no_gauss:
+        gauss_result, outputs["gauss_lnl"] = run_gauss(nb, lib, _lib, dev, rank, dist, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs, dist, rank)
     cube_result = None
     if args.cube_size > 0 or args.scale_cube != "0x0" or args.full_cube:
-        del d_params, d_lnl, flush
+        del d_params, d_lnl, flush, outputs
         torch.cuda.empty_cache()
         cube_result = run_cube_fit(nb, args, rank, world, dev, dist)
     if rank != 0:
@@ -412,9 +423,10 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
-def run_gauss(nb, lib, _lib, dev, rank, dist):
+def run_gauss(nb, lib, _lib, dev, rank, dist, n_it):
     """Secondary metric (BASELINE configs[4]): Gaussian model, 8 components over 4096 channels, 2^20 vectors per
-    GPU against 256 pixels (replicated data, disjoint vector slices); device-resident evals/s, max over ranks."""
+    GPU against 256 pixels (replicated data, disjoint vector slices); device-resident evals/s over `n_it` timed
+    launches, max over ranks.  Returns (result line or None off rank 0, device lnL of the last launch)."""
     import torch
     from nestfit_b200.parallel import max_over_ranks
     B, n_chan, ncomp, n_pix = 1 << 20, 4096, 8, 256
@@ -441,7 +453,6 @@ def run_gauss(nb, lib, _lib, dev, rank, dist):
     if dist is not None:
         dist.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    n_it = 10
     e0.record()
     for _ in range(n_it):
         launch()
@@ -450,10 +461,11 @@ def run_gauss(nb, lib, _lib, dev, rank, dist):
     ms = max_over_ranks(e0.elapsed_time(e1) / n_it, dist, device=f"cuda:{dev}")
     blk.close()
     if rank != 0:
-        return None
+        return None, d_l
     world = 1 if dist is None else dist.get_world_size()
     return {"metric": "Gaussian loglike evals/s (8-comp, 4096 ch)", "value": world * B / (ms * 1e-3), "unit": "evals/s",
-            "ms_per_launch": ms, "vectors_per_gpu": B, "windowed_gaussians_per_eval": WORK_GAUSS_MODEL, "scaling": "weak"}
+            "ms_per_launch": ms, "launches": n_it, "vectors_per_gpu": B, "windowed_gaussians_per_eval": WORK_GAUSS_MODEL,
+            "scaling": "weak"}, d_l
 
 
 def _shared_cube(nb, shape, ncomp_max, noise_grad, seed, dev, rank, dist, tag):
@@ -685,6 +697,32 @@ def cube_cpu_baseline(stack, ut, shape, nbest_gpu):
             "nbest_agrees_with_gpu": float((nb_cpu == nbest_gpu[lon, lat]).mean())}
 
 
+DUMP_LIMIT_BYTES = 64_000_000 - 4096      # 64 MB of files in all, npy headers included
+
+
+def dump_outputs(dirname, tensors, dist, rank):
+    """Write each device output as DIR/<name>.npy in float64 from rank 0: the slices of all ranks in rank order,
+    i.e. everything the callers of the multi-GPU path receive.  An array that would take the files past 64 MB
+    is replaced by a fixed sample of it: the entries at the sorted indices `default_rng(0).choice(n, k)`."""
+    import torch
+    arrays = {}
+    for name, t in tensors.items():
+        if dist is not None:
+            parts = [torch.empty_like(t) for _ in range(dist.get_world_size())]
+            dist.all_gather(parts, t)
+            t = torch.cat(parts)
+        arrays[name] = t.double().cpu().numpy()
+    if rank != 0:
+        return
+    k = DUMP_LIMIT_BYTES // (8 * len(arrays))
+    out = Path(dirname)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        if a.size > k:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, k, replace=False))]
+        np.save(out / f"{name}.npy", a)
+
+
 def _with_device(nb, dev):
     """PixelBlock / PriorTransformer helpers default to device 0; bind to `dev`."""
     if dev == 0:
@@ -820,7 +858,13 @@ def main():
     ap.add_argument("--blocks-per-gpu", type=int, default=8, help="over-decomposition of the multi-GPU cube fit")
     ap.add_argument("--concurrent-blocks", type=int, default=2,
                     help="groups of blocks a rank keeps in flight (host threads / streams)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the lnL arrays of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed: not available with --impl reference")
     if args.gpus > 1 and "RANK" not in os.environ:
         # convenience: re-launch one process per GPU (the driver does this itself)
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",

@@ -103,10 +103,18 @@ def is_built():
     return True
 
 
+def sources_present():
+    """True when the reference's sources can be read at REF; a path the user may not enter counts as absent."""
+    try:
+        return (REF / "nestfit" / "core" / "core.pyx").is_file() and os.access(REF, os.R_OK | os.X_OK)
+    except OSError:
+        return False
+
+
 def build(force=False):
     if is_built() and not force:
         return True
-    if not (REF / "nestfit" / "core" / "core.pyx").exists():
+    if not sources_present():
         return False
     work = Path(tempfile.mkdtemp(prefix="nestfit_ref_build_"))
     try:
