@@ -18,7 +18,8 @@
  *   - `nnhp_predict` / `DiazenyliumRunner.c_loglikelihood`   nestfit/models/diazenylium.pyx:140-158,206-215
  *       -> nf_n2hp_predict / nf_n2hp_loglike
  *   - `AmmoniaSpectrum.__init__`, `Spectrum.__init__`        nestfit/models/ammonia.pyx:245-277, nestfit/core/core.pyx:488-520
- *       -> nf_pixels_create (+ nf_pixels_null_lnz)
+ *       -> nf_pixels_create (+ nf_pixels_null_lnz); spectra on their own axes and lengths
+ *          (one Runner each, run_multinest per Runner) -> nf_pixels_create_axes
  *   - `PriorTransformer.c_transform`                         nestfit/core/core.pyx:459-476
  *       -> nf_priors_create + nf_prior_transform
  *   - MultiNest `run(...)` + `LogLike`/`dumper` callbacks    nestfit/core/cmultinest.pxd:5-33,
@@ -93,6 +94,20 @@ int nf_pixels_create_from_device(int device, int model, int64_t n_pix, int n_spe
                                  const double *nu_chan, const int *trans_id,
                                  const double *rest_freq, const float *data_dev,
                                  const double *noise_dev, nf_pixels **out);
+/* Same, but every (pixel, spectrum) has its own uniform ascending axis
+ * x_j = nu_min[p][s] + j*nu_chan[p][s] and its own channel count
+ * 2 <= n_chan[p][s] <= n_chan_max <= 65535: a catalogue of pointed
+ * observations, or spectra cut from cubes with different set-ups.  `data` is
+ * [n_pix][n_spec][n_chan_max]; channels past a spectrum's own n_chan are
+ * stored as zero whatever the caller passed there.  The transitions
+ * `trans_id[n_spec]` are shared by all pixels; the Gaussian model (n_spec = 1)
+ * takes one `rest_freq[n_pix]` per pixel.  The *_loglike[_host] entry points
+ * work unchanged on such a block; predictions need a pixel per vector and go
+ * through nf_predict_pix[_host] (the *_predict[_host] calls return NF_EINVAL). */
+int nf_pixels_create_axes(int device, int model, int64_t n_pix, int n_spec, int n_chan_max,
+                          const double *nu_min, const double *nu_chan, const int *n_chan,
+                          const int *trans_id, const double *rest_freq,
+                          const void *data, int dtype, const double *noise, nf_pixels **out);
 int nf_pixels_free(nf_pixels *px);
 /* null-model evidence per pixel, -sum_s sum_j d^2/(2 sigma_s^2)
  * (core.pyx:518-520, ammonia.pyx:411-415) -> host double[n_pix]. */
@@ -126,6 +141,13 @@ int nf_n2hp_predict(const nf_pixels *px, const void *params_dev, int param_dtype
                     int64_t B, int ncomp, float *pred_dev, void *stream);
 int nf_gauss_predict(const nf_pixels *px, const void *params_dev, int param_dtype,
                      int64_t B, int ncomp, float *pred_dev, void *stream);
+/* Model spectra of any block's model, vector b on the axes of pixel
+ * pix_of_vec_dev[b] (required): pred_dev [B][n_spec][n_chan] FP32, n_chan
+ * being the block's longest spectrum; channels past a spectrum's own length
+ * are 0.  `flags` as for NH3 (ignored by the other models). */
+int nf_predict_pix(const nf_pixels *px, const void *params_dev, int param_dtype,
+                   const int32_t *pix_of_vec_dev, int64_t B, int ncomp, int flags,
+                   float *pred_dev, void *stream);
 
 /* ---- host-buffer entry points (the call a reference-side binding makes) -- */
 /* params_host [B][ndim] of param_dtype, pix_of_vec_host may be NULL (then
@@ -150,6 +172,9 @@ int nf_n2hp_loglike_host(const nf_pixels *px, const void *params_host, int param
                          int64_t B, int ncomp, double *lnL_host);
 int nf_n2hp_predict_host(const nf_pixels *px, const void *params_host, int param_dtype,
                          int64_t B, int ncomp, float *pred_host);
+int nf_predict_pix_host(const nf_pixels *px, const void *params_host, int param_dtype,
+                        const int32_t *pix_of_vec_host, int64_t B, int ncomp, int flags,
+                        float *pred_host);
 
 /* ---- prior transform ---------------------------------------------------- */
 int nf_priors_create(int device, const nf_prior_desc *priors, int n_prior,

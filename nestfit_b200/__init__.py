@@ -13,7 +13,7 @@ from .models.ammonia import amm_predict, AmmoniaSpectrum, AmmoniaRunner  # noqa:
 from .models.gaussian import gauss_predict, GaussianRunner  # noqa: F401
 from .models.diazenylium import nnhp_predict, DiazenyliumSpectrum, DiazenyliumRunner  # noqa: F401
 from .prior_constructors import get_irdc_priors, get_synth_priors  # noqa: F401
-from .sampler import NestedSamplingBatch, Dumper, run_multinest  # noqa: F401
+from .sampler import NestedSamplingBatch, Dumper, run_multinest, run_multinest_batch  # noqa: F401
 from .store import HdfStore, MemGroup  # noqa: F401
 from .main import (  # noqa: F401
     NoiseMap, NoiseMapUniform, DataCube, CubeStack, CubeFitter, get_multiproc_indices, get_block_indices,

@@ -55,6 +55,7 @@ _SIGNATURES = {
     "nf_device_count": ([_PI], _I),
     "nf_pixels_create": ([_I, _I, _I64, _I, _I, _VP, _VP, _VP, _VP, _VP, _I, _VP, C.POINTER(_VP)], _I),
     "nf_pixels_create_from_device": ([_I, _I, _I64, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, C.POINTER(_VP)], _I),
+    "nf_pixels_create_axes": ([_I, _I, _I64, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _I, _VP, C.POINTER(_VP)], _I),
     "nf_pixels_free": ([_VP], _I),
     "nf_pixels_null_lnz": ([_VP, _VP], _I),
     "nf_nh3_loglike": ([_VP, _VP, _I, _VP, _I64, _I64, _I, _I, _VP, _VP], _I),
@@ -69,6 +70,8 @@ _SIGNATURES = {
     "nf_gauss_loglike_host": ([_VP, _VP, _I, _VP, _I64, _I64, _I, _VP], _I),
     "nf_nh3_predict_host": ([_VP, _VP, _I, _I64, _I, _I, _VP], _I),
     "nf_gauss_predict_host": ([_VP, _VP, _I, _I64, _I, _VP], _I),
+    "nf_predict_pix": ([_VP, _VP, _I, _VP, _I64, _I, _I, _VP, _VP], _I),
+    "nf_predict_pix_host": ([_VP, _VP, _I, _VP, _I64, _I, _I, _VP], _I),
     "nf_priors_create": ([_I, _VP, _I, _VP, _I, _VP, _I64, _I, C.POINTER(_VP)], _I),
     "nf_priors_free": ([_VP], _I),
     "nf_prior_transform": ([_VP, _VP, _I64, _I, _VP], _I),

@@ -62,49 +62,55 @@ struct DeviceGuard {
 
 #define NF_CUDA(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) return (int)e__; } while (0)
 
+// Constants of one spectrum of n channels on the axis x_j = nu_min + j nu_chan; `t` is its transition id (hyperfine
+// models) and `rest_freq` its rest frequency (Gaussian model, may be NULL otherwise).
+int fill_spec_meta(int model, int n, double nu_min, double nu_chan, int t, const double *rest_freq, NfSpecMeta &m)
+{
+    std::memset(&m, 0, sizeof(m));
+    if (!(nu_chan > 0.0) || !std::isfinite(nu_min)) return NF_EINVAL;       // core.pyx:504
+    m.nu_min = nu_min;
+    m.nu_chan = nu_chan;
+    m.inv_chan = 1.0 / nu_chan;
+    const double x_last = nu_min + (double)(n - 1) * nu_chan;
+    m.T0_first = NF_H * nu_min / NF_KB;
+    m.T0_last = NF_H * x_last / NF_KB;
+    const double nm1 = n > 1 ? (double)(n - 1) : 1.0;
+    m.t0a = (float)m.T0_first;
+    m.t0b = (float)((m.T0_last - m.T0_first) / nm1);
+    m.tbg0 = 1.0 / std::expm1(m.T0_first / NF_TCMB);
+    m.tbg1 = (1.0 / std::expm1(m.T0_last / NF_TCMB) - m.tbg0) / nm1;
+    if (model == NF_MODEL_NH3) {
+        if (t < 1 || t > NF_NH3_NTRANS) return NF_EINVAL;                   // ammonia.pyx:268
+        m.J = t;
+        m.para = (t % 3) != 0;
+        m.nu0 = kNu[t - 1];
+        m.line_off = kOff[t - 1];
+        m.nlines = kOff[t] - kOff[t - 1];
+        m.fracterm = NF_CCMS * NF_CCMS * kEa[t - 1] / (8.0 * M_PI * m.nu0 * m.nu0);
+        m.width_c = NF_CKMS / (m.nu0 * std::sqrt(2.0 * M_PI));
+        m.hnu_k = NF_H * m.nu0 / NF_KB;
+    } else if (model == NF_MODEL_N2HP) {
+        if (t < 1 || t > NF_N2HP_NTRANS) return NF_EINVAL;                  // diazenylium.pyx:128
+        m.J = t;
+        m.nu0 = kNuN2hp[t - 1];
+        m.line_off = NF_NH3_NLINES_TOTAL + kOffN2hp[t - 1];                 // flat line list of nf_nh3.cu
+        m.nlines = kOffN2hp[t] - kOffN2hp[t - 1];
+        m.hnu_k = NF_H * m.nu0 / NF_KB;
+    } else {
+        if (!rest_freq || !(*rest_freq > 0.0)) return NF_EINVAL;
+        m.nu0 = *rest_freq;
+        m.nlines = 1;
+    }
+    return NF_OK;
+}
+
 int fill_meta(nf_pixels *px, const double *nu_min, const double *nu_chan, const int *trans_id,
               const double *rest_freq)
 {
-    const int n = px->n_chan;
     for (int s = 0; s < px->n_spec; ++s) {
-        NfSpecMeta &m = px->spec[s];
-        std::memset(&m, 0, sizeof(m));
-        if (!(nu_chan[s] > 0.0) || !std::isfinite(nu_min[s])) return NF_EINVAL;   // core.pyx:504
-        m.nu_min = nu_min[s];
-        m.nu_chan = nu_chan[s];
-        m.inv_chan = 1.0 / nu_chan[s];
-        const double x_last = nu_min[s] + (double)(n - 1) * nu_chan[s];
-        m.T0_first = NF_H * nu_min[s] / NF_KB;
-        m.T0_last = NF_H * x_last / NF_KB;
-        const double nm1 = n > 1 ? (double)(n - 1) : 1.0;
-        m.t0a = (float)m.T0_first;
-        m.t0b = (float)((m.T0_last - m.T0_first) / nm1);
-        m.tbg0 = 1.0 / std::expm1(m.T0_first / NF_TCMB);
-        m.tbg1 = (1.0 / std::expm1(m.T0_last / NF_TCMB) - m.tbg0) / nm1;
-        if (px->model == NF_MODEL_NH3) {
-            const int t = trans_id ? trans_id[s] : 0;
-            if (t < 1 || t > NF_NH3_NTRANS) return NF_EINVAL;                   // ammonia.pyx:268
-            m.J = t;
-            m.para = (t % 3) != 0;
-            m.nu0 = kNu[t - 1];
-            m.line_off = kOff[t - 1];
-            m.nlines = kOff[t] - kOff[t - 1];
-            m.fracterm = NF_CCMS * NF_CCMS * kEa[t - 1] / (8.0 * M_PI * m.nu0 * m.nu0);
-            m.width_c = NF_CKMS / (m.nu0 * std::sqrt(2.0 * M_PI));
-            m.hnu_k = NF_H * m.nu0 / NF_KB;
-        } else if (px->model == NF_MODEL_N2HP) {
-            const int t = trans_id ? trans_id[s] : 0;
-            if (t < 1 || t > NF_N2HP_NTRANS) return NF_EINVAL;                  // diazenylium.pyx:128
-            m.J = t;
-            m.nu0 = kNuN2hp[t - 1];
-            m.line_off = NF_NH3_NLINES_TOTAL + kOffN2hp[t - 1];                 // flat line list of nf_nh3.cu
-            m.nlines = kOffN2hp[t] - kOffN2hp[t - 1];
-            m.hnu_k = NF_H * m.nu0 / NF_KB;
-        } else {
-            if (!rest_freq || !(rest_freq[s] > 0.0)) return NF_EINVAL;
-            m.nu0 = rest_freq[s];
-            m.nlines = 1;
-        }
+        const int rc = fill_spec_meta(px->model, px->n_chan, nu_min[s], nu_chan[s], trans_id ? trans_id[s] : 0,
+                                      rest_freq ? rest_freq + s : nullptr, px->spec[s]);
+        if (rc != NF_OK) return rc;
     }
     return NF_OK;
 }
@@ -160,6 +166,30 @@ int upload_noise(nf_pixels *px, const double *noise_host)
     }
     NF_CUDA(cudaMemcpy(px->inv2s2, inv.data(), nrow * sizeof(double), cudaMemcpyHostToDevice));
     return NF_OK;
+}
+
+// raw host rows [n_pix * n_spec][n_chan] of dtype -> device scratch -> padded FP32 rows, in bounded pieces
+int upload_host_rows(nf_pixels *px, const void *data, int dtype)
+{
+    const int n_chan = px->n_chan;
+    const size_t esz = dtype == NF_F64 ? 8 : 4;
+    const int64_t rows = px->n_pix * px->n_spec;
+    int64_t piece = (int64_t)((size_t)64 << 20) / ((size_t)n_chan * esz);
+    if (piece < 1) piece = 1;
+    if (piece > rows) piece = rows;
+    void *scratch = nullptr;
+    cudaError_t e = cudaMalloc(&scratch, (size_t)piece * n_chan * esz);
+    for (int64_t r0 = 0; e == cudaSuccess && r0 < rows; r0 += piece) {
+        const int64_t nr = rows - r0 < piece ? rows - r0 : piece;
+        e = cudaMemcpy(scratch, (const unsigned char *)data + (size_t)r0 * n_chan * esz,
+                       (size_t)nr * n_chan * esz, cudaMemcpyHostToDevice);
+        if (e == cudaSuccess)
+            e = nf_launch_pack_rows(scratch, dtype == NF_F64, px->data + (size_t)r0 * px->n_pad, nr, n_chan,
+                                    px->n_pad, 0);
+        if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    }
+    if (scratch) cudaFree(scratch);
+    return (int)e;
 }
 
 int finish_pixels(nf_pixels *px)
@@ -251,7 +281,7 @@ int make_args(const nf_pixels *px, const void *params, int param_dtype, const in
     a->inv2s2 = px->inv2s2;
     a->d2chunk = use_data ? px->d2chunk : nullptr;
     a->params = params;
-    a->pix_of_vec = use_data ? pix_of_vec : nullptr;
+    a->pix_of_vec = (use_data || px->pixmeta) ? pix_of_vec : nullptr;   // predictions on per-pixel axes need the map
     a->vecs_per_pix = vecs_per_pix > 0 ? vecs_per_pix : 1;
     a->B = B;
     a->pix_stride = (int64_t)px->n_spec * px->n_pad;
@@ -265,6 +295,7 @@ int make_args(const nf_pixels *px, const void *params, int param_dtype, const in
     a->cold = (flags & NF_FLAG_COLD) != 0;
     a->lte = (flags & NF_FLAG_LTE) != 0;
     for (int s = 0; s < px->n_spec; ++s) a->spec[s] = px->spec[s];
+    a->pixmeta = px->pixmeta;
     return NF_OK;
 }
 
@@ -376,6 +407,7 @@ int run_host(const nf_pixels *px, int model, const void *params_host, int param_
             a.data = px->data + (b0 / a.vecs_per_pix) * a.pix_stride;
             a.inv2s2 = px->inv2s2 + (b0 / a.vecs_per_pix) * px->n_spec;
             a.d2chunk = px->d2chunk + (b0 / a.vecs_per_pix) * px->n_spec * (px->n_pad / 32);
+            if (px->pixmeta) a.pixmeta = px->pixmeta + (b0 / a.vecs_per_pix) * px->n_spec;
         }
         NF_STEP(cudaEventRecord(ev0[slot], st));
         NF_STEP(launch_model(model, a, st));
@@ -451,26 +483,55 @@ int nf_pixels_create(int device, int model, int64_t n_pix, int n_spec, int n_cha
     for (int64_t i = 0; i < n_pix * n_spec; ++i)
         if (!(noise[i] > 0.0)) { nf_pixels_free(px); return NF_EINVAL; }
     rc = upload_noise(px, noise);
-    // raw rows -> device scratch -> padded FP32 rows, in bounded pieces
-    const size_t esz = dtype == NF_F64 ? 8 : 4;
+    if (rc == NF_OK) rc = upload_host_rows(px, data, dtype);
+    if (rc == NF_OK) rc = finish_pixels(px);
+    if (rc != NF_OK) { nf_pixels_free(px); return rc; }
+    *out = px;
+    return NF_OK;
+}
+
+int nf_pixels_create_axes(int device, int model, int64_t n_pix, int n_spec, int n_chan_max, const double *nu_min,
+                          const double *nu_chan, const int *n_chan, const int *trans_id, const double *rest_freq,
+                          const void *data, int dtype, const double *noise, nf_pixels **out)
+{
+    if (!out) return NF_EINVAL;
+    *out = nullptr;
+    if (!data || !noise || !n_chan || !nu_min || !nu_chan || (dtype != NF_F32 && dtype != NF_F64)) return NF_EINVAL;
+    if (n_pix <= 0 || n_spec <= 0 || n_spec > NF_MAX_SPEC || n_chan_max < 2 || n_chan_max > 65535) return NF_EINVAL;
+    if (model == NF_MODEL_GAUSS && (n_spec != 1 || !rest_freq)) return NF_EINVAL;
     const int64_t rows = n_pix * n_spec;
-    int64_t piece = (int64_t)((size_t)64 << 20) / ((size_t)n_chan * esz);
-    if (piece < 1) piece = 1;
-    if (piece > rows) piece = rows;
-    void *scratch = nullptr;
-    cudaError_t e = cudaSuccess;
-    if (rc == NF_OK) e = cudaMalloc(&scratch, (size_t)piece * n_chan * esz);
-    for (int64_t r0 = 0; rc == NF_OK && e == cudaSuccess && r0 < rows; r0 += piece) {
-        const int64_t nr = rows - r0 < piece ? rows - r0 : piece;
-        e = cudaMemcpy(scratch, (const unsigned char *)data + (size_t)r0 * n_chan * esz,
-                       (size_t)nr * n_chan * esz, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess)
-            e = nf_launch_pack_rows(scratch, dtype == NF_F64, px->data + (size_t)r0 * px->n_pad, nr, n_chan,
-                                    px->n_pad, 0);
-        if (e == cudaSuccess) e = cudaDeviceSynchronize();
-    }
-    if (scratch) cudaFree(scratch);
-    if (rc == NF_OK && e != cudaSuccess) rc = (int)e;
+    std::vector<NfPixSpecMeta> meta((size_t)rows);
+    for (int64_t p = 0; p < n_pix; ++p)
+        for (int sp = 0; sp < n_spec; ++sp) {
+            const int64_t r = p * n_spec + sp;
+            const int n = n_chan[r];
+            if (n < 2 || n > n_chan_max || !(noise[r] > 0.0)) return NF_EINVAL;       // core.pyx:502
+            std::memset(&meta[(size_t)r], 0, sizeof(NfPixSpecMeta));
+            meta[(size_t)r].n_chan = n;
+            const int rc = fill_spec_meta(model, n, nu_min[r], nu_chan[r], trans_id ? trans_id[sp] : 0,
+                                          model == NF_MODEL_GAUSS ? rest_freq + p : nullptr, meta[(size_t)r].m);
+            if (rc != NF_OK) return rc;
+        }
+    // channels past a spectrum's own end are zero in HBM, whatever the caller left there: the null evidence, the
+    // per-chunk sums of d^2 and the residual pass then need no channel counts
+    const size_t esz = dtype == NF_F64 ? 8 : 4, row_bytes = (size_t)n_chan_max * esz;
+    std::vector<unsigned char> rows_zf((size_t)rows * row_bytes);
+    std::memcpy(rows_zf.data(), data, rows_zf.size());
+    for (int64_t r = 0; r < rows; ++r)
+        std::memset(rows_zf.data() + (size_t)r * row_bytes + (size_t)n_chan[r] * esz, 0,
+                    (size_t)(n_chan_max - n_chan[r]) * esz);
+    DeviceGuard g(device);
+    if (!g.ok) return NF_ENODEV;
+    nf_pixels *px = nullptr;
+    int rc = pixels_alloc(device, model, n_pix, n_spec, n_chan_max, nu_min, nu_chan, trans_id, rest_freq, &px);
+    if (rc != NF_OK) return rc;
+    for (int sp = 0; sp < n_spec; ++sp) px->spec[sp] = meta[(size_t)sp].m;    // pixel 0: the shared transitions
+    cudaError_t e = cudaMalloc(&px->pixmeta, (size_t)rows * sizeof(NfPixSpecMeta));
+    if (e == cudaSuccess)
+        e = cudaMemcpy(px->pixmeta, meta.data(), (size_t)rows * sizeof(NfPixSpecMeta), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) rc = (int)e;
+    if (rc == NF_OK) rc = upload_noise(px, noise);
+    if (rc == NF_OK) rc = upload_host_rows(px, rows_zf.data(), dtype);
     if (rc == NF_OK) rc = finish_pixels(px);
     if (rc != NF_OK) { nf_pixels_free(px); return rc; }
     *out = px;
@@ -513,6 +574,7 @@ int nf_pixels_free(nf_pixels *px)
     if (px->inv2s2) cudaFree(px->inv2s2);
     if (px->null_lnz) cudaFree(px->null_lnz);
     if (px->d2chunk) cudaFree(px->d2chunk);
+    if (px->pixmeta) cudaFree(px->pixmeta);
     for (int i = 0; i < NF_HOST_SLOTS; ++i) {
         if (px->stage_dev[i]) cudaFree(px->stage_dev[i]);
         if (px->stage_host[i]) cudaFreeHost(px->stage_host[i]);
@@ -547,7 +609,7 @@ int nf_nh3_loglike(const nf_pixels *px, const void *params_dev, int param_dtype,
 int nf_nh3_predict(const nf_pixels *px, const void *params_dev, int param_dtype, int64_t B, int ncomp,
                    int flags, float *pred_dev, void *stream)
 {
-    if (!px || px->model != NF_MODEL_NH3 || !pred_dev) return NF_EINVAL;
+    if (!px || px->model != NF_MODEL_NH3 || !pred_dev || px->pixmeta) return NF_EINVAL;
     NfLikeArgs a;
     int rc = make_args(px, params_dev, param_dtype, nullptr, 1, B, ncomp, flags, nullptr, pred_dev, false, &a);
     if (rc != NF_OK) return rc;
@@ -569,7 +631,7 @@ int nf_n2hp_loglike(const nf_pixels *px, const void *params_dev, int param_dtype
 int nf_n2hp_predict(const nf_pixels *px, const void *params_dev, int param_dtype, int64_t B, int ncomp,
                     float *pred_dev, void *stream)
 {
-    if (!px || px->model != NF_MODEL_N2HP || !pred_dev) return NF_EINVAL;
+    if (!px || px->model != NF_MODEL_N2HP || !pred_dev || px->pixmeta) return NF_EINVAL;
     NfLikeArgs a;
     int rc = make_args(px, params_dev, param_dtype, nullptr, 1, B, ncomp, 0, nullptr, pred_dev, false, &a);
     if (rc != NF_OK) return rc;
@@ -588,7 +650,7 @@ int nf_n2hp_loglike_host(const nf_pixels *px, const void *params_host, int param
 int nf_n2hp_predict_host(const nf_pixels *px, const void *params_host, int param_dtype, int64_t B, int ncomp,
                          float *pred_host)
 {
-    if (!pred_host) return NF_EINVAL;
+    if (!pred_host || (px && px->pixmeta)) return NF_EINVAL;
     return run_host(px, NF_MODEL_N2HP, params_host, param_dtype, nullptr, 1, B, ncomp, 0, nullptr, pred_host);
 }
 
@@ -607,7 +669,7 @@ int nf_gauss_loglike(const nf_pixels *px, const void *params_dev, int param_dtyp
 int nf_gauss_predict(const nf_pixels *px, const void *params_dev, int param_dtype, int64_t B, int ncomp,
                      float *pred_dev, void *stream)
 {
-    if (!px || px->model != NF_MODEL_GAUSS || !pred_dev) return NF_EINVAL;
+    if (!px || px->model != NF_MODEL_GAUSS || !pred_dev || px->pixmeta) return NF_EINVAL;
     NfLikeArgs a;
     int rc = make_args(px, params_dev, param_dtype, nullptr, 1, B, ncomp, 0, nullptr, pred_dev, false, &a);
     if (rc != NF_OK) return rc;
@@ -635,15 +697,32 @@ int nf_gauss_loglike_host(const nf_pixels *px, const void *params_host, int para
 int nf_nh3_predict_host(const nf_pixels *px, const void *params_host, int param_dtype, int64_t B, int ncomp,
                         int flags, float *pred_host)
 {
-    if (!pred_host) return NF_EINVAL;
+    if (!pred_host || (px && px->pixmeta)) return NF_EINVAL;
     return run_host(px, NF_MODEL_NH3, params_host, param_dtype, nullptr, 1, B, ncomp, flags, nullptr, pred_host);
 }
 
 int nf_gauss_predict_host(const nf_pixels *px, const void *params_host, int param_dtype, int64_t B, int ncomp,
                           float *pred_host)
 {
-    if (!pred_host) return NF_EINVAL;
+    if (!pred_host || (px && px->pixmeta)) return NF_EINVAL;
     return run_host(px, NF_MODEL_GAUSS, params_host, param_dtype, nullptr, 1, B, ncomp, 0, nullptr, pred_host);
+}
+
+int nf_predict_pix(const nf_pixels *px, const void *params_dev, int param_dtype, const int32_t *pix_of_vec_dev,
+                   int64_t B, int ncomp, int flags, float *pred_dev, void *stream)
+{
+    if (!px || !pred_dev || !pix_of_vec_dev) return NF_EINVAL;
+    NfLikeArgs a;
+    int rc = make_args(px, params_dev, param_dtype, pix_of_vec_dev, 1, B, ncomp, flags, nullptr, pred_dev, false, &a);
+    if (rc != NF_OK) return rc;
+    return run_device(px, a, stream);
+}
+
+int nf_predict_pix_host(const nf_pixels *px, const void *params_host, int param_dtype, const int32_t *pix_of_vec_host,
+                        int64_t B, int ncomp, int flags, float *pred_host)
+{
+    if (!px || !pred_host || !pix_of_vec_host) return NF_EINVAL;
+    return run_host(px, px->model, params_host, param_dtype, pix_of_vec_host, 1, B, ncomp, flags, nullptr, pred_host);
 }
 
 int nf_last_call_stats(double *kernel_ms, int64_t *n_launches)

@@ -42,6 +42,14 @@ struct NfSpecMeta {
     int para;           // para (K % 3 != 0) or ortho
 };
 
+// One (pixel, spectrum) of a block whose pixels have their own axes: the spectrum's constants and its own channel
+// count (rows are zero past it up to the block's n_chan).
+struct NfPixSpecMeta {
+    NfSpecMeta m;
+    int n_chan;
+    int pad_;
+};
+
 #define NF_HOST_SLOTS 3         // chunks in flight in a host-buffer call (ring of streams and staging buffers)
 
 struct nf_pixels {
@@ -53,7 +61,8 @@ struct nf_pixels {
     double *inv2s2;                 // [n_pix][n_spec]  1/(2 sigma^2)
     double *null_lnz;               // [n_pix]
     float *d2chunk;                 // [n_pix][n_spec][n_pad/32]  sum of d^2 over each 32-channel chunk
-    NfSpecMeta spec[NF_MAX_SPEC];
+    NfSpecMeta spec[NF_MAX_SPEC];   // per-pixel axes: pixel 0's (the transitions are shared by all pixels)
+    NfPixSpecMeta *pixmeta;         // [n_pix][n_spec] on the device when every pixel has its own axes, else NULL
     // pipelined host-call resources (one host-buffer call at a time per block: guarded by host_mu)
     std::mutex *host_mu;
     cudaStream_t streams[NF_HOST_SLOTS];
@@ -94,6 +103,8 @@ struct NfLikeArgs {
     int stage;                  // hyperfine kernel: the tile's pixel is staged in shared memory (set by the launcher)
     int nkey;                   // hyperfine kernel: line keys per component (set by the launcher)
     NfSpecMeta spec[NF_MAX_SPEC];
+    const NfPixSpecMeta *pixmeta;   // per-pixel axes [n_pix][n_spec] (NULL: every pixel uses spec[]); n_chan is then the
+                                    // longest spectrum and pred rows are that long
 };
 
 // launchers (nf_model.cu)

@@ -80,9 +80,18 @@ __device__ __noinline__ float4 gauss_row4_global(const float *p)
     return make_float4(__ldg(p), __ldg(p + 32), __ldg(p + 64), __ldg(p + 96));
 }
 
+// channels of the spectrum of pixel pix
+template <bool PIXAX>
+__device__ __forceinline__ int gauss_nchan_of(const NfLikeArgs &a, int64_t pix)
+{
+    if constexpr (PIXAX) return a.pixmeta[pix].n_chan;
+    else return a.n_chan;
+}
+
 // WRITE_PRED = false: log-likelihood against the pixel's data (a.data, a.lnL);
 // WRITE_PRED = true : model spectra only (a.pred), no data are read.
-template <bool WRITE_PRED, typename PT>
+// PIXAX: every pixel has its own axis and channel count (a.pixmeta); a.n_chan is the longest spectrum.
+template <bool WRITE_PRED, typename PT, bool PIXAX>
 __global__ void __launch_bounds__(NF_THREADS, NF_GAUSS_MIN_CTAS)
 nf_gauss_kernel(const __grid_constant__ NfLikeArgs a)
 {
@@ -115,14 +124,17 @@ nf_gauss_kernel(const __grid_constant__ NfLikeArgs a)
     const int ncomp = a.ncomp;
     const int ndim = 3 * ncomp;
     const int nchunks = (a.n_chan + 127) >> 7;       // 128-channel chunks (rows are padded to a multiple of 128)
-    const NfSpecMeta &sm = a.spec[0];
-    const double nu_min = sm.nu_min, inv_chan = sm.inv_chan, f0 = sm.nu0;
+    const NfSpecMeta &sm = a.spec[0];                  // PIXAX: the vector's pixel's entry of a.pixmeta instead
+    const double nu_min_b = sm.nu_min, inv_chan_b = sm.inv_chan, f0_b = sm.nu0;
     const float lane_f = (float)lane;
 
     for (int64_t b = b0 + warp; b < b0 + tile && b < B; b += NF_WARPS_PER_CTA) {
         const int64_t pbase = b * ndim;
         int64_t pix = 0;
-        if (have_data) pix = a.pix_of_vec ? (int64_t)__ldg(a.pix_of_vec + b) : b / a.vecs_per_pix;
+        if (have_data || PIXAX) pix = a.pix_of_vec ? (int64_t)__ldg(a.pix_of_vec + b) : b / a.vecs_per_pix;
+        const NfPixSpecMeta *pm = PIXAX ? a.pixmeta + pix : nullptr;
+        const double nu_min = PIXAX ? pm->m.nu_min : nu_min_b, inv_chan = PIXAX ? pm->m.inv_chan : inv_chan_b;
+        const double f0 = PIXAX ? pm->m.nu0 : f0_b;
 
         // ---- set-up, lanes <-> components (gaussian.pyx:25-46) ----
         int lo = 0, hi = 0;
@@ -141,9 +153,9 @@ nf_gauss_kernel(const __grid_constant__ NfLikeArgs a)
             // NaN to 0, so non-finite parameters end up with an empty window.
             lo = __double2int_rd((rel - cut) * inv_chan);
             hi = __double2int_rd((rel + cut) * inv_chan);
-            on = act && !(hi < 0 || lo > a.n_chan - 1);         // gaussian.pyx:41
+            on = act && !(hi < 0 || lo > gauss_nchan_of<PIXAX>(a, pix) - 1);   // gaussian.pyx:41
             lo = max(lo, 0);
-            hi = min(hi, a.n_chan - 1);
+            hi = min(hi, gauss_nchan_of<PIXAX>(a, pix) - 1);
             on = on && hi > lo;                                 // loop j in [lo, hi)
             GaussRec r;
             r.a = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -250,10 +262,10 @@ nf_gauss_kernel(const __grid_constant__ NfLikeArgs a)
                         const int j0 = (int)__uint_as_float(ent.y);
                         if (WRITE_PRED) {
                             const int j = j0 + lane;
-                            if (j < a.n_chan) prow[j] = m0;
-                            if (j + 32 < a.n_chan) prow[j + 32] = m1;
-                            if (j + 64 < a.n_chan) prow[j + 64] = m2;
-                            if (j + 96 < a.n_chan) prow[j + 96] = m3;
+                            if (j < gauss_nchan_of<PIXAX>(a, pix)) prow[j] = m0;
+                            if (j + 32 < gauss_nchan_of<PIXAX>(a, pix)) prow[j + 32] = m1;
+                            if (j + 64 < gauss_nchan_of<PIXAX>(a, pix)) prow[j + 64] = m2;
+                            if (j + 96 < gauss_nchan_of<PIXAX>(a, pix)) prow[j + 96] = m3;
                         } else {
                             float q0, q1, q2, q3;
                             if (staged) {
@@ -287,10 +299,10 @@ nf_gauss_kernel(const __grid_constant__ NfLikeArgs a)
     if (!data_ready) mbar_wait(bar, 0);
 }
 
-template <bool WP, typename PT>
+template <bool WP, typename PT, bool PIXAX>
 static cudaError_t gauss_launch_one(const NfLikeArgs &a, cudaStream_t st)
 {
-    auto kern = nf_gauss_kernel<WP, PT>;
+    auto kern = nf_gauss_kernel<WP, PT, PIXAX>;
     const size_t smem = 128 + (((size_t)a.n_pad * 4 + 127) / 128) * 128 + sizeof(GaussScratch) * NF_WARPS_PER_CTA;
     if (smem > 227 * 1024) return cudaErrorInvalidConfiguration;
     cudaError_t e = nf_ensure_dyn_smem((const void *)kern, smem);
@@ -302,13 +314,19 @@ static cudaError_t gauss_launch_one(const NfLikeArgs &a, cudaStream_t st)
     return cudaGetLastError();
 }
 
+template <bool PIXAX>
+static cudaError_t gauss_launch_ax(const NfLikeArgs &a, cudaStream_t st)
+{
+    const bool wp = a.pred != nullptr;
+    if (a.param_f64)
+        return wp ? gauss_launch_one<true, double, PIXAX>(a, st) : gauss_launch_one<false, double, PIXAX>(a, st);
+    return wp ? gauss_launch_one<true, float, PIXAX>(a, st) : gauss_launch_one<false, float, PIXAX>(a, st);
+}
+
 cudaError_t nf_launch_gauss(const NfLikeArgs &a, cudaStream_t st)
 {
     if (a.ncomp < 1 || a.ncomp > NF_MAX_NCOMP_GAUSS || a.n_spec != 1) return cudaErrorInvalidValue;
-    const bool wp = a.pred != nullptr;
-    if (a.param_f64)
-        return wp ? gauss_launch_one<true, double>(a, st) : gauss_launch_one<false, double>(a, st);
-    return wp ? gauss_launch_one<true, float>(a, st) : gauss_launch_one<false, float>(a, st);
+    return a.pixmeta ? gauss_launch_ax<true>(a, st) : gauss_launch_ax<false>(a, st);
 }
 
 // ---- pixel-block helpers ----------------------------------------------------

@@ -130,10 +130,30 @@ __device__ double nh3_iemtex(double x)
 #define NH3_BK_F ((float)(NF_HK * NF_BROT))
 #define NH3_CK_F ((float)(NF_HK * (NF_CROT - NF_BROT)))
 
+// ---- per-pixel axes (PIXAX) ------------------------------------------------------
+// Spectrum s of pixel pix: the block's shared constants, or that pixel's own entry in HBM.
+template <bool PIXAX>
+__device__ __forceinline__ const NfSpecMeta &nh3_spec_of(const NfLikeArgs &a, int64_t pix, int s)
+{
+    if constexpr (PIXAX) return a.pixmeta[pix * a.n_spec + s].m;
+    else return a.spec[s];
+}
+template <bool PIXAX>
+__device__ __forceinline__ int nh3_nchan_of(const NfLikeArgs &a, int64_t pix, int s)
+{
+    if constexpr (PIXAX) return a.pixmeta[pix * a.n_spec + s].n_chan;
+    else return a.n_chan;
+}
+__device__ __forceinline__ int64_t nh3_pix_of(const NfLikeArgs &a, int64_t b)
+{
+    return a.pix_of_vec ? (int64_t)__ldg(a.pix_of_vec + b) : b / a.vecs_per_pix;
+}
+
 // ---- S: batched set-up, lanes <-> (vector, component, spectrum) -----------------
 // MODEL 0: NH3 (voff, trot, tex, ntot, sigm, orth; ammonia.pyx:326-361);
 // MODEL 1: N2H+ (voff, tex, ltau, sigm; diazenylium.pyx:140-154).
-template <int MODEL, int NC, typename PT, typename SC>
+// PIXAX: every lane reads the axis of its own vector's pixel.
+template <int MODEL, int NC, bool PIXAX, typename PT, typename SC>
 __device__ __noinline__ void nh3_setup_batch(const NfLikeArgs &a, SC &sc, int64_t bb, int nb, int lane)
 {
     const int n_spec = a.n_spec;
@@ -143,7 +163,8 @@ __device__ __noinline__ void nh3_setup_batch(const NfLikeArgs &a, SC &sc, int64_
     const int c = r / n_spec, s = r - c * n_spec;
     const bool valid = kk < nb;
     const int64_t pbase = (bb + (valid ? kk : 0)) * ((MODEL == 0 ? 6 : 4) * NC);
-    const NfSpecMeta &sm = a.spec[s];
+    const int64_t pix = PIXAX ? nh3_pix_of(a, bb + (valid ? kk : 0)) : 0;
+    const NfSpecMeta &sm = nh3_spec_of<PIXAX>(a, pix, s);
     const double voff = ld_param<PT>(a.params, pbase + 0 * NC + c);
     double tex, sigm, tau_main;
     if constexpr (MODEL == 1) {
@@ -194,7 +215,7 @@ __device__ __noinline__ void nh3_setup_batch(const NfLikeArgs &a, SC &sc, int64_
     // T_B amplitude T0_j * (G(T0_j/tex) - tbg_j), hyperfine.pyx:106-113, as the max of two
     // lines in j: the reference's G is a convex piecewise-linear table, so this reproduces
     // the table lerp -- including a knot inside the band -- without per-channel look-ups.
-    const double nm1 = (double)(a.n_chan - 1);
+    const double nm1 = (double)(nh3_nchan_of<PIXAX>(a, pix, s) - 1);
     const double xL = sm.T0_first / tex, xR = sm.T0_last / tex;
     const double dxdj = (xR - xL) / nm1;
     double aL, bL, aR, bR;
@@ -320,7 +341,9 @@ __device__ __forceinline__ void blk_m_add(uint32_t ma, const float (&val)[8])
     sts128(ma + BLK_PLANE, v);
 }
 
-template <int MODEL, int NC, bool WRITE_PRED, typename PT>
+// PIXAX: every pixel has its own axes and channel counts (a.pixmeta); a.n_chan is the longest spectrum, and the
+// super-blocks and the residual run to it (data and model are zero past a spectrum's own end).
+template <int MODEL, int NC, bool WRITE_PRED, typename PT, bool PIXAX>
 __global__ void __launch_bounds__(NF_THREADS, (NC <= 3 ? BLK_MINCTA : 2))
 nf_nh3_kernel(const __grid_constant__ NfLikeArgs a)
 {
@@ -378,17 +401,18 @@ nf_nh3_kernel(const __grid_constant__ NfLikeArgs a)
 
     for (int64_t bb = b0 + (int64_t)warp * vpw; bb < bw_end; bb += vb) {
         const int nb = (int)min((int64_t)vb, bw_end - bb);
-        nh3_setup_batch<MODEL, NC, PT, Scratch>(a, sc, bb, nb, lane);
+        nh3_setup_batch<MODEL, NC, PIXAX, PT, Scratch>(a, sc, bb, nb, lane);
         __syncwarp();
 
         for (int k = 0; k < nb; ++k) {
             const int64_t b = bb + k;
             int64_t pix = 0;
-            if (have_data) pix = a.pix_of_vec ? (int64_t)__ldg(a.pix_of_vec + b) : b / a.vecs_per_pix;
+            if (have_data || PIXAX) pix = a.pix_of_vec ? (int64_t)__ldg(a.pix_of_vec + b) : b / a.vecs_per_pix;
             const bool staged = have_data && pix == pix0;
             double lnl = 0.0;
             for (int s = 0; s < n_spec; ++s) {
-                const NfSpecMeta &sm = a.spec[s];
+                const NfSpecMeta &sm = nh3_spec_of<PIXAX>(a, pix, s);
+                const int n_own = nh3_nchan_of<PIXAX>(a, pix, s);     // channels of this spectrum
                 const int NL = sm.nlines, nitems_l = NC * NL;
                 // ---- L: line records, lanes <-> (component, line) flattened; counts of super-block 0 ----
                 for (int idx = lane; idx < NC * BLK_STRIDE; idx += 32) cw[idx] = 0u;
@@ -414,10 +438,10 @@ nf_nh3_kernel(const __grid_constant__ NfLikeArgs a)
                         // and maps NaN to 0, so non-finite parameters end up with an empty window.
                         int lo = __double2int_rd((rel - cut) * inv_chan);
                         int hi = __double2int_rd((rel + cut) * inv_chan);
-                        const bool inband = !(hi < 0 || lo > a.n_chan - 1);   // hyperfine.pyx:88
+                        const bool inband = !(hi < 0 || lo > n_own - 1);      // hyperfine.pyx:88
                         const bool below = hi < 0;
                         lo = max(lo, 0);
-                        hi = min(hi, a.n_chan - 1);
+                        hi = min(hi, n_own - 1);
                         const bool on = inband && hi > lo;                    // loop j in [lo, hi)
                         // block keys, ascending in the (frequency-sorted) line index.  An in-band line with an
                         // empty window keeps a nominal one-channel extent so that both keys stay sorted.
@@ -627,7 +651,8 @@ nf_nh3_kernel(const __grid_constant__ NfLikeArgs a)
                         const int nreal = min(BLK_SB * 8, a.n_chan - ch0);
                         for (int j = lane; j < nreal; j += 32) {
                             const int bq = j >> 3;
-                            row[ch0 + j] = sc.m[(blk_m_off(bq) + ((j >> 2) & 1) * BLK_PLANE) / 4 + (j & 3)];
+                            const float mv = sc.m[(blk_m_off(bq) + ((j >> 2) & 1) * BLK_PLANE) / 4 + (j & 3)];
+                            row[ch0 + j] = (PIXAX && ch0 + j >= n_own) ? 0.0f : mv;   // past the spectrum's end
                         }
                         __syncwarp();
                         for (int idx = lane; idx < BLK_M_BYTES / 4; idx += 32) sc.m[idx] = 0.0f;
@@ -687,7 +712,7 @@ static size_t nh3_smem_bytes(const NfLikeArgs &a, int nwarps)
     return 128 + data + ((size_t)NC * a.npair * 24 + (size_t)NC * a.nkey * sizeof(short2) + sizeof(BlkScratch<NC>)) * nwarps;
 }
 
-template <int MODEL, int NC, bool WP, typename PT>
+template <int MODEL, int NC, bool WP, typename PT, bool PIXAX>
 static cudaError_t nh3_launch_one(const NfLikeArgs &a0, cudaStream_t st)
 {
     NfLikeArgs a = a0;
@@ -695,7 +720,7 @@ static cudaError_t nh3_launch_one(const NfLikeArgs &a0, cudaStream_t st)
     for (int s = 0; s < a.n_spec; ++s) max_lines = a.spec[s].nlines > max_lines ? a.spec[s].nlines : max_lines;
     a.npair = (max_lines + 1) & ~1;                            // records per component (even: 16-byte aligned arrays)
     a.nkey = a.n_chan > BLK_SB * 8 ? ((max_lines + 3) & ~3) : 0;   // line keys are only re-read by later super-blocks
-    auto kern = nf_nh3_kernel<MODEL, NC, WP, PT>;
+    auto kern = nf_nh3_kernel<MODEL, NC, WP, PT, PIXAX>;
     // the tile's pixel is staged in shared memory by one bulk copy; rows too long for that are read from HBM / L2
     a.stage = WP ? 0 : 1;
     size_t smem = nh3_smem_bytes<NC>(a, NH3_WARPS);
@@ -713,13 +738,20 @@ static cudaError_t nh3_launch_one(const NfLikeArgs &a0, cudaStream_t st)
     return cudaGetLastError();
 }
 
-template <int MODEL, int NC>
-static cudaError_t nh3_launch_nc(const NfLikeArgs &a, cudaStream_t st)
+template <int MODEL, int NC, bool PIXAX>
+static cudaError_t nh3_launch_ax(const NfLikeArgs &a, cudaStream_t st)
 {
     const bool wp = a.pred != nullptr;
     if (a.param_f64)
-        return wp ? nh3_launch_one<MODEL, NC, true, double>(a, st) : nh3_launch_one<MODEL, NC, false, double>(a, st);
-    return wp ? nh3_launch_one<MODEL, NC, true, float>(a, st) : nh3_launch_one<MODEL, NC, false, float>(a, st);
+        return wp ? nh3_launch_one<MODEL, NC, true, double, PIXAX>(a, st)
+                  : nh3_launch_one<MODEL, NC, false, double, PIXAX>(a, st);
+    return wp ? nh3_launch_one<MODEL, NC, true, float, PIXAX>(a, st) : nh3_launch_one<MODEL, NC, false, float, PIXAX>(a, st);
+}
+
+template <int MODEL, int NC>
+static cudaError_t nh3_launch_nc(const NfLikeArgs &a, cudaStream_t st)
+{
+    return a.pixmeta ? nh3_launch_ax<MODEL, NC, true>(a, st) : nh3_launch_ax<MODEL, NC, false>(a, st);
 }
 
 cudaError_t nf_launch_nh3(const NfLikeArgs &a, cudaStream_t st)

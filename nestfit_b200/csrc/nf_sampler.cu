@@ -1118,6 +1118,7 @@ int score(nf_sampler *s, double *params, const int32_t *pix, int64_t vpp, int64_
     a.cold = (s->flags & NF_FLAG_COLD) != 0; a.lte = (s->flags & NF_FLAG_LTE) != 0;
     a.tile_vecs = (int)(vpp > 0 ? vpp : 0);     // a CTA tile never straddles the proposals of two runs (pixels)
     for (int k = 0; k < px->n_spec; ++k) a.spec[k] = px->spec[k];
+    a.pixmeta = px->pixmeta;
     NS_CUDA(px->model == NF_MODEL_NH3 ? nf_launch_nh3(a, s->stream)
             : px->model == NF_MODEL_N2HP ? nf_launch_n2hp(a, s->stream) : nf_launch_gauss(a, s->stream));
     s->launches += 2;

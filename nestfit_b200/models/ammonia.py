@@ -23,6 +23,8 @@ class AmmoniaSpectrum(HyperfineSpectrum):
 
 
 def _block_from_spectra(spectra, device=0):
+    if len({s.size for s in spectra}) > 1:      # spectra of different lengths: each on its own axis
+        return PixelBlock.from_spectra("ammonia", [spectra], device=device)
     xarrs = [s.xarr for s in spectra]
     data = np.stack([s.data for s in spectra])[None, :, :]
     noise = np.array([[s.noise for s in spectra]])
@@ -44,6 +46,7 @@ def amm_predict(s, params, cold=False, lte=False):
 
 class AmmoniaRunner(Runner):
     """Likelihood operator over one pixel's NH3 spectra (ammonia.pyx:369-447)."""
+    model_name = 'ammonia'
 
     def __init__(self, spectra, utrans, ncomp=1, cold=False, lte=False):
         assert ncomp > 0
@@ -89,9 +92,10 @@ class AmmoniaRunner(Runner):
             ncomp = self.ncomp
             shape = params.shape[0]
             raise ValueError(f'Invalid shape for ncomp={ncomp}: {shape}')
-        pred = self._block.predict(params.reshape(1, -1), self.ncomp, cold=self.cold, lte=self.lte)[0]
+        pix = [0] if self._block.per_pixel_axes else None
+        pred = self._block.predict(params.reshape(1, -1), self.ncomp, cold=self.cold, lte=self.lte, pix_of_vec=pix)[0]
         for i, spec in enumerate(self.spectra):
-            spec.pred[:] = pred[i]
+            spec.pred[:] = pred[i, :spec.size]
 
 
 # Aliases and metadata consumed by the store (ammonia.pyx:451-489, main.py:369-377)

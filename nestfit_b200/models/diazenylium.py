@@ -22,6 +22,8 @@ class DiazenyliumSpectrum(HyperfineSpectrum):
 
 
 def _block_from_spectra(spectra, device=0):
+    if len({s.size for s in spectra}) > 1:      # spectra of different lengths: each on its own axis
+        return PixelBlock.from_spectra("diazenylium", [spectra], device=device)
     xarrs = [s.xarr for s in spectra]
     data = np.stack([s.data for s in spectra])[None, :, :]
     noise = np.array([[s.noise for s in spectra]])
@@ -42,6 +44,7 @@ def nnhp_predict(s, params):
 
 class DiazenyliumRunner(Runner):
     """Likelihood operator over one pixel's N2H+ spectra (diazenylium.pyx:161-232)."""
+    model_name = 'diazenylium'
 
     def __init__(self, spectra, utrans, ncomp=1):
         assert ncomp > 0
@@ -83,9 +86,10 @@ class DiazenyliumRunner(Runner):
             ncomp = self.ncomp
             shape = params.shape[0]
             raise ValueError(f'Invalid shape for ncomp={ncomp}: {shape}')
-        pred = self._block.predict(params.reshape(1, -1), self.ncomp)[0]
+        pix = [0] if self._block.per_pixel_axes else None
+        pred = self._block.predict(params.reshape(1, -1), self.ncomp, pix_of_vec=pix)[0]
         for i, spec in enumerate(self.spectra):
-            spec.pred[:] = pred[i]
+            spec.pred[:] = pred[i, :spec.size]
 
 
 # Aliases and metadata consumed by the store (diazenylium.pyx:235-272, main.py:369-377)

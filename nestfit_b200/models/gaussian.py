@@ -26,6 +26,7 @@ def gauss_predict(s, params):
 
 class GaussianRunner(Runner):
     """Likelihood operator for one spectrum (gaussian.pyx:57-112)."""
+    model_name = 'gaussian'
 
     def __init__(self, spectrum, utrans, ncomp=1):
         assert ncomp > 0

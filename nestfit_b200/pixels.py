@@ -5,7 +5,9 @@ It is the batched counterpart of the reference's per-pixel ``Spectrum`` /
 ``AmmoniaSpectrum`` objects (nestfit/core/core.pyx:486-520,
 nestfit/models/ammonia.pyx:244-277): the cube's ``data[lon, lat, chan]`` slab
 (nestfit/main.py:152) is uploaded once and every likelihood call references
-pixels by index.
+pixels by index.  ``PixelBlock.from_spectra`` uploads spectra that do not form a
+cube -- a catalogue of pointed observations, where every (pixel, spectrum) has
+its own axis and length.
 """
 import ctypes as C
 
@@ -14,7 +16,13 @@ import numpy as np
 from . import _lib
 
 
+_MODELS = {"ammonia": _lib.NF_MODEL_NH3, "gaussian": _lib.NF_MODEL_GAUSS, "diazenylium": _lib.NF_MODEL_N2HP}
+_N_MODEL = {_lib.NF_MODEL_NH3: 6, _lib.NF_MODEL_N2HP: 4, _lib.NF_MODEL_GAUSS: 3}
+
+
 class PixelBlock:
+    per_pixel_axes = False
+
     def __init__(self, model, xarrs, data, noise, trans_ids=None, rest_freq=None, device=0):
         """
         model     : 'ammonia' | 'gaussian' | 'diazenylium'
@@ -27,8 +35,7 @@ class PixelBlock:
         from .core import check_uniform_axis
         lib = _lib.load()
         self.model_name = model
-        self.model = {"ammonia": _lib.NF_MODEL_NH3, "gaussian": _lib.NF_MODEL_GAUSS,
-                      "diazenylium": _lib.NF_MODEL_N2HP}[model]
+        self.model = _MODELS[model]
         xarrs = [np.ascontiguousarray(x, dtype=np.float64) for x in xarrs]
         self.n_spec = len(xarrs)
         self.n_chan = int(xarrs[0].shape[0])
@@ -65,7 +72,70 @@ class PixelBlock:
                                         _lib.ptr(data), dtype, _lib.ptr(noise), C.byref(out)),
                    "nf_pixels_create")
         self.handle = out
-        self.n_model = {_lib.NF_MODEL_NH3: 6, _lib.NF_MODEL_N2HP: 4, _lib.NF_MODEL_GAUSS: 3}[self.model]
+        self.n_model = _N_MODEL[self.model]
+
+    @classmethod
+    def from_spectra(cls, model, spectra, device=0):
+        """Block in which every (pixel, spectrum) has its own uniform ascending axis and length.
+
+        spectra[p] is pixel p's list of Spectrum-like objects (``xarr``, ``data``, ``noise``, ``trans_id``; the
+        Gaussian model takes one spectrum per pixel and its ``rest_freq``).  All pixels have the same number of
+        spectra and the same transitions.  ``n_chan`` is then [n_pix, n_spec] and ``n_chan_max`` its maximum;
+        ``predict`` needs ``pix_of_vec`` and returns rows of ``n_chan_max`` channels, zero past each spectrum's end.
+        """
+        from .core import check_uniform_axis
+        lib = _lib.load()
+        self = cls.__new__(cls)
+        self.model_name = model
+        self.model = _MODELS[model]
+        self.per_pixel_axes = True
+        spectra = [list(sp) for sp in spectra]
+        n_pix = len(spectra)
+        if n_pix == 0:
+            raise ValueError("from_spectra needs at least one pixel")
+        n_spec = len(spectra[0])
+        if n_spec < 1 or any(len(sp) != n_spec for sp in spectra):
+            raise ValueError("every pixel must have the same number of spectra")
+        if n_spec > _lib.NF_MAX_SPEC:
+            raise ValueError(f"at most {_lib.NF_MAX_SPEC} spectra per pixel")
+        if self.model == _lib.NF_MODEL_GAUSS and n_spec != 1:
+            raise ValueError("the Gaussian model takes one spectrum per pixel")
+        n_chan = np.array([[int(np.asarray(s.xarr).shape[0]) for s in sp] for sp in spectra], dtype=np.int32)
+        n_chan_max = int(n_chan.max())
+        nu_min = np.empty((n_pix, n_spec))
+        nu_chan = np.empty((n_pix, n_spec))
+        noise = np.empty((n_pix, n_spec))
+        data = np.zeros((n_pix, n_spec, n_chan_max))
+        for p, sp in enumerate(spectra):
+            for k, s in enumerate(sp):
+                x = np.ascontiguousarray(s.xarr, dtype=np.float64)
+                check_uniform_axis(x)
+                d = np.asarray(s.data, dtype=np.float64)
+                if d.shape != x.shape:
+                    raise ValueError(f"pixel {p} spectrum {k}: data and axis lengths differ")
+                nu_min[p, k], nu_chan[p, k] = x[0], x[1] - x[0]
+                noise[p, k] = s.noise
+                data[p, k, :x.shape[0]] = d
+        tid = rf = None
+        if self.model in (_lib.NF_MODEL_NH3, _lib.NF_MODEL_N2HP):
+            tid = np.array([s.trans_id for s in spectra[0]], dtype=np.int32)
+            if any([s.trans_id for s in sp] != list(tid) for sp in spectra):
+                raise ValueError("all pixels of a block must have the same transitions")
+        else:
+            rf = np.array([sp[0].rest_freq for sp in spectra], dtype=np.float64)
+        self.n_pix, self.n_spec = n_pix, n_spec
+        self.n_chan, self.n_chan_max = n_chan, n_chan_max
+        self.xarrs = None
+        self.trans_ids, self.rest_freq = tid, rf
+        self.device = device
+        self.n_model = _N_MODEL[self.model]
+        out = C.c_void_p()
+        _lib.check(lib.nf_pixels_create_axes(device, self.model, n_pix, n_spec, n_chan_max, _lib.ptr(nu_min),
+                                             _lib.ptr(nu_chan), _lib.ptr(n_chan), _lib.ptr(tid), _lib.ptr(rf),
+                                             _lib.ptr(data), _lib.NF_F64, _lib.ptr(noise), C.byref(out)),
+                   "nf_pixels_create_axes")
+        self.handle = out
+        return self
 
     def close(self):
         if getattr(self, "handle", None):
@@ -125,16 +195,34 @@ class PixelBlock:
         _lib.check(rc, "loglike")
         return out
 
-    def predict(self, params, ncomp, cold=False, lte=False):
-        """Model spectra for params [B, n_model*ncomp] -> float32 [B, n_spec, n_chan]."""
+    def predict(self, params, ncomp, cold=False, lte=False, pix_of_vec=None):
+        """Model spectra for params [B, n_model*ncomp] -> float32 [B, n_spec, n_chan].
+
+        With ``pix_of_vec`` (required on a block from ``from_spectra``) vector b is synthesised on the axes of pixel
+        pix_of_vec[b]; rows then have ``n_chan_max`` channels and are zero past each spectrum's own length."""
         lib = _lib.load()
         params, dt = self._params(params)
         if params.ndim != 2 or params.shape[1] != self.n_model * ncomp:
             raise ValueError(f'Invalid shape for ncomp={ncomp}: {params.shape}')
         B = params.shape[0]
+        if self.per_pixel_axes and pix_of_vec is None:
+            raise ValueError("a block with per-pixel axes needs pix_of_vec to predict")
+        flags = (_lib.NF_FLAG_COLD if cold else 0) | (_lib.NF_FLAG_LTE if lte else 0)
+        if pix_of_vec is not None:
+            pv = np.ascontiguousarray(pix_of_vec, dtype=np.int32)
+            if pv.shape != (B,):
+                raise ValueError("pix_of_vec must have one entry per vector")
+            if B and (pv.min() < 0 or pv.max() >= self.n_pix):
+                raise ValueError("pix_of_vec out of range")
+            n_row = self.n_chan_max if self.per_pixel_axes else self.n_chan
+            out = np.empty((B, self.n_spec, n_row), dtype=np.float32)
+            if self.model != _lib.NF_MODEL_NH3:
+                flags = 0
+            _lib.check(lib.nf_predict_pix_host(self.handle, _lib.ptr(params), dt, _lib.ptr(pv), B, ncomp, flags,
+                                               _lib.ptr(out)), "predict")
+            return out
         out = np.empty((B, self.n_spec, self.n_chan), dtype=np.float32)
         if self.model == _lib.NF_MODEL_NH3:
-            flags = (_lib.NF_FLAG_COLD if cold else 0) | (_lib.NF_FLAG_LTE if lte else 0)
             rc = lib.nf_nh3_predict_host(self.handle, _lib.ptr(params), dt, B, ncomp, flags, _lib.ptr(out))
         elif self.model == _lib.NF_MODEL_N2HP:
             rc = lib.nf_n2hp_predict_host(self.handle, _lib.ptr(params), dt, B, ncomp, _lib.ptr(out))

@@ -250,3 +250,132 @@ def run_multinest(runner, dumper, IS=False, mmodal=True, ceff=False, nlive=400, 
         dumper.n_samples = int(res["n_samples"][0])
     ns.close()
     return res
+
+
+def _runner_spectra(runner):
+    """The spectra of one runner's pixel (the Gaussian runner holds a single one)."""
+    spectra = getattr(runner, "spectra", None)
+    return [runner.spectrum] if spectra is None else list(spectra)
+
+
+def _check_batch(runners, dumpers, nlive, tol, efr, maxiter, max_runs_per_batch, nClsPar):
+    """Argument checks of run_multinest_batch; touch no device."""
+    if len(runners) == 0:
+        raise ValueError("run_multinest_batch needs at least one runner")
+    r0 = runners[0]
+    if getattr(r0, "model_name", None) is None:
+        raise ValueError(f"{type(r0).__name__} is not a runner of this package")
+
+    def trans(r):
+        return tuple(int(s.trans_id) for s in _runner_spectra(r))
+
+    for i, r in enumerate(runners[1:], start=1):
+        for what, a, b in (("class", type(r), type(r0)), ("ncomp", r.ncomp, r0.ncomp),
+                           ("number of spectra", r.n_spec, r0.n_spec), ("transition ids", trans(r), trans(r0)),
+                           ("cold", bool(getattr(r, "cold", False)), bool(getattr(r0, "cold", False))),
+                           ("lte", bool(getattr(r, "lte", False)), bool(getattr(r0, "lte", False)))):
+            if a != b:
+                raise ValueError(f"runner {i} differs from runner 0 in its {what}: {a!r} != {b!r}")
+        if r.utrans is not r0.utrans:
+            raise ValueError(f"runner {i} has another prior transformer than runner 0")
+    n = len(runners)
+    if dumpers is not None and len(dumpers) != n:
+        raise ValueError(f"{len(dumpers)} dumpers for {n} runners")
+    nl = np.asarray(nlive)
+    if nl.ndim > 1 or (nl.ndim == 1 and nl.shape[0] != n):
+        raise ValueError(f"nlive must be a scalar or one value per runner ({n}), got shape {nl.shape}")
+    if not np.all(nl > 0):
+        raise ValueError("nlive must be positive")
+    if not tol > 0:
+        raise ValueError("tol must be positive")
+    if not 0 < efr <= 1:
+        raise ValueError("efr must lie in (0, 1]")
+    if maxiter < 0:
+        raise ValueError("maxiter must not be negative")
+    if max_runs_per_batch < 1:
+        raise ValueError("max_runs_per_batch must be at least 1")
+    if nClsPar is not None and nClsPar > r0.n_params:
+        raise ValueError('Number of clustering parameters must be less than total.')
+
+
+def run_multinest_batch(runners, dumpers=None, nlive=400, tol=0.5, efr=0.3, seed=-1, maxiter=int(1e6), n_prop=32,
+                        max_runs_per_batch=16384, **multinest_switches):
+    """Batched form of ``run_multinest``: fits every runner's pixel in lock-step on the device.
+
+    The runners may come from anywhere -- a catalogue of pointed observations, spectra cut from several cubes --
+    and each spectrum keeps its own axis and length: their spectra are uploaded as one block with per-pixel axes
+    (``PixelBlock.from_spectra``) and fitted by ``NestedSamplingBatch`` in batches of at most
+    ``max_runs_per_batch`` runs.  All runners must share class, ``ncomp``, number of spectra, transition ids,
+    ``cold`` / ``lte`` and prior transformer (checked, with ``ValueError``, before the device is touched).
+
+    For each runner it sets ``runner.run_lnZ`` and writes into ``dumpers[i]`` (None: no products) what
+    ``run_multinest(runners[i], dumpers[i])`` writes, with that runner's own ``null_lnZ`` and ``n_chan_tot``.
+    ``nlive`` is a scalar or one value per runner.  Truncated runs are flagged (``truncated``) but not repeated.
+    MultiNest-only switches are accepted and ignored, as in ``run_multinest``.  Returns the per-runner result
+    arrays (``lnZ``, ``lnZ_err``, ``max_loglike``, ``n_samples``, ``n_iter``, ``n_evals``, ``bestfit``,
+    ``mapfit``, ``truncated``) in runner order.
+
+    Choosing the number of components stays the caller's loop, as with the reference: one call per ncomp over
+    the sources that are still improving::
+
+        best = np.zeros(len(catalogue), dtype=int)      # 0: nothing detected
+        lnZ_best = np.empty(len(catalogue))
+        active = np.arange(len(catalogue))
+        for ncomp in (1, 2, 3):
+            batch = [AmmoniaRunner(catalogue[i], utrans, ncomp=ncomp) for i in active]
+            run_multinest_batch(batch)
+            lnZ = np.array([r.run_lnZ for r in batch])
+            ref = np.array([r.null_lnZ for r in batch]) if ncomp == 1 else lnZ_best[active]
+            better = lnZ - ref > lnZ_thresh                # e.g. lnZ_thresh = 11
+            best[active[better]] = ncomp
+            lnZ_best[active[better]] = lnZ[better]
+            active = active[better]
+            if active.size == 0:
+                break
+    """
+    from .pixels import PixelBlock
+    runners = list(runners)
+    _check_batch(runners, dumpers, nlive, tol, efr, maxiter, max_runs_per_batch, multinest_switches.get("nClsPar"))
+    n = len(runners)
+    r0 = runners[0]
+    dumpers = [None] * n if dumpers is None else list(dumpers)
+    nlive = np.broadcast_to(np.asarray(nlive, dtype=np.int32), (n,))
+    cold, lte = bool(getattr(r0, "cold", False)), bool(getattr(r0, "lte", False))
+    block = PixelBlock.from_spectra(r0.model_name, [_runner_spectra(r) for r in runners])
+    parts = []
+    try:
+        for k, b0 in enumerate(range(0, n, max_runs_per_batch)):
+            sel = np.arange(b0, min(n, b0 + max_runs_per_batch))
+            bseed = seed if seed is None or seed < 0 else seed + k
+            ns = NestedSamplingBatch(block, r0.utrans, r0.ncomp, pix_ids=sel, nlive=nlive[sel], tol=tol, efr=efr,
+                                     n_prop=n_prop, seed=bseed, max_iter=maxiter, cold=cold, lte=lte)
+            try:
+                res = ns.run()
+                dump = [dumpers[i] is not None and not dumpers[i].no_dump for i in sel]
+                if any(dump):          # the posteriors of the whole batch in one device pass and one copy
+                    prod = ns.products_all(marginals=False, posteriors=True)
+                    off, pool = prod["row_offsets"], prod["posteriors"]
+                for j, i in enumerate(sel):
+                    runner, dumper = runners[i], dumpers[i]
+                    runner.run_lnZ = float(res["lnZ"][j])
+                    if dump[j]:
+                        post = pool[off[j]:off[j + 1]].astype(np.float64)
+                        attrs, dsets = run_products(
+                            r0.ncomp, ns.ndim, int(ns.nlive[j]), runner.null_lnZ, runner.n_chan_tot, post,
+                            res["lnZ"][j], res["lnZ_err"][j], res["max_loglike"][j], res["bestfit"][j],
+                            res["mapfit"][j], n_iter=res["n_iter"][j], n_evals=res["n_evals"][j],
+                            truncated=res["truncated"][j])
+                        dumper.append_attributes(**attrs)
+                        dumper.append_datasets(**dsets)
+                    if dumper is not None:
+                        dumper.n_calls = getattr(dumper, "n_calls", 0) + 1
+                        dumper.n_samples = int(res["n_samples"][j])
+                parts.append(res)
+            finally:
+                ns.close()
+    finally:
+        block.close()
+    out = {key: np.concatenate([p[key] for p in parts]) for key, v in parts[0].items() if isinstance(v, np.ndarray)}
+    out["lock_iters"] = sum(p["lock_iters"] for p in parts)
+    out["launches"] = sum(p["launches"] for p in parts)
+    return out
