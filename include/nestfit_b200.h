@@ -58,6 +58,11 @@ enum { NF_FLAG_COLD = 1, NF_FLAG_LTE = 2 };
 #define NF_MAX_SPEC 6       /* spectra (transitions) scored together per pixel */
 #define NF_MAX_NCOMP_NH3 4  /* velocity components of the fused NH3 kernel      */
 #define NF_MAX_NCOMP_GAUSS 32
+/* Widest spectrum the hyperfine models (NH3, N2H+) accept, as (nu_last - nu_first) / nu_first (about 240 km/s).
+ * Their kernel makes the brightness amplitude T0 (G(T0/tex) - tbg) linear in the channel; the error of that grows
+ * with the square of the band, and up to this width it stays inside 1e-5 of a spectrum's peak for tex down to
+ * 2.8 K.  The pixel-block constructors return NF_EINVAL for a wider hyperfine spectrum. */
+#define NF_MAX_BAND_FRAC 8e-4
 
 typedef struct nf_pixels nf_pixels; /* opaque: a block of pixels resident in HBM */
 typedef struct nf_priors nf_priors; /* opaque: a prior plan resident in HBM      */

@@ -19,6 +19,7 @@ NF_FLAG_COLD, NF_FLAG_LTE = 1, 2
 NF_MAX_SPEC = 6
 NF_MAX_NCOMP_NH3 = 4
 NF_MAX_NCOMP_GAUSS = 32
+NF_MAX_BAND_FRAC = 8e-4      # widest hyperfine spectrum, (nu_last - nu_first) / nu_first
 
 
 class NfError(RuntimeError):

@@ -72,6 +72,7 @@ int fill_spec_meta(int model, int n, double nu_min, double nu_chan, int t, const
     m.nu_chan = nu_chan;
     m.inv_chan = 1.0 / nu_chan;
     const double x_last = nu_min + (double)(n - 1) * nu_chan;
+    if (model != NF_MODEL_GAUSS && !((x_last - nu_min) / nu_min <= NF_MAX_BAND_FRAC)) return NF_EINVAL;
     m.T0_first = NF_H * nu_min / NF_KB;
     m.T0_last = NF_H * x_last / NF_KB;
     const double nm1 = n > 1 ? (double)(n - 1) : 1.0;

@@ -100,7 +100,7 @@ struct NfLikeArgs {
     int cold, lte;
     int tile_vecs;              // parameter vectors per CTA tile (0 -> NF_TILE_VECS)
     int npair;                  // hyperfine kernel: line records per component (set by the launcher)
-    int stage;                  // hyperfine kernel: the tile's pixel is staged in shared memory (set by the launcher)
+    int stage;                  // the tile's pixel is staged in shared memory (set by the launcher)
     int nkey;                   // hyperfine kernel: line keys per component (set by the launcher)
     NfSpecMeta spec[NF_MAX_SPEC];
     const NfPixSpecMeta *pixmeta;   // per-pixel axes [n_pix][n_spec] (NULL: every pixel uses spec[]); n_chan is then the

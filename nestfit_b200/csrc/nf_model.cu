@@ -7,7 +7,8 @@
 //   + {0, 32, 64, 96} (packed FP32x2 across channel pairs): most chunks are touched by one component, so
 //   four channels per lane spread the per-chunk work (record fetch, residual) over more terms.
 // A CTA (8 warps) works on a tile of consecutive vectors; the pixel of the tile's first vector
-// is staged once in shared memory with a TMA bulk copy (cp.async.bulk + mbarrier).  Components
+// is staged once in shared memory with a TMA bulk copy (cp.async.bulk + mbarrier), unless the row is too long to
+// fit (more than 51840 channels): every pixel is then read from HBM / L2.  Components
 // are unordered and have unequal widths: per super-block of 32 chunks the (chunk, component) pairs that
 // overlap are compacted into a flat, channel-ordered work list (lanes <-> chunks: every lane collects the
 // components covering its chunk from the other lanes' chunk masks, a warp scan places its entries), and the
@@ -73,8 +74,8 @@ __constant__ uint32_t g_lsb_rec_off[32] = {
     18 * 32, 6 * 32, 11 * 32, 5 * 32, 10 * 32, 9 * 32};
 static_assert(sizeof(GaussRec) == 32, "g_lsb_rec_off is scaled by the record size");
 
-// Four channels of a pixel row that is not the CTA's staged pixel (rare: tiles straddling two pixels).  Kept out
-// of line so that the compiler does not predicate these loads into the common path.
+// Four channels of a pixel row that is not the CTA's staged pixel (tiles straddling two pixels, rows too long to
+// stage).  Kept out of line so that the compiler does not predicate these loads into the common path.
 __device__ __noinline__ float4 gauss_row4_global(const float *p)
 {
     return make_float4(__ldg(p), __ldg(p + 32), __ldg(p + 64), __ldg(p + 96));
@@ -98,7 +99,7 @@ nf_gauss_kernel(const __grid_constant__ NfLikeArgs a)
     extern __shared__ __align__(128) unsigned char smem_raw[];
     uint64_t *bar = reinterpret_cast<uint64_t *>(smem_raw);
     float *sdata = reinterpret_cast<float *>(smem_raw + 128);
-    const int data_floats = a.n_pad;                      // one spectrum per pixel (gaussian.pyx:94-96)
+    const int data_floats = a.stage ? a.n_pad : 0;       // one spectrum per pixel (gaussian.pyx:94-96)
     GaussScratch *scr_all = reinterpret_cast<GaussScratch *>(smem_raw + 128 + (((size_t)data_floats * 4 + 127) / 128) * 128);
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -111,15 +112,15 @@ nf_gauss_kernel(const __grid_constant__ NfLikeArgs a)
     const int64_t B = a.B_dev ? min(a.B, (int64_t)__ldg(a.B_dev)) : a.B;
     if (b0 >= B) return;
     constexpr bool have_data = !WRITE_PRED;
-    int64_t pix0 = 0;
-    if (have_data) {
+    int64_t pix0 = -1;
+    if (have_data && a.stage) {
         pix0 = a.pix_of_vec ? (int64_t)__ldg(a.pix_of_vec + b0) : b0 / a.vecs_per_pix;
         if (tid == 0) mbar_init(bar, 1);
         __syncthreads();
         if (tid == 0)
             tma_load_1d(sdata, a.data + pix0 * a.pix_stride, (uint32_t)(data_floats * 4), bar);
     }
-    bool data_ready = !have_data;
+    bool data_ready = !(have_data && a.stage);
 
     const int ncomp = a.ncomp;
     const int ndim = 3 * ncomp;
@@ -300,10 +301,20 @@ nf_gauss_kernel(const __grid_constant__ NfLikeArgs a)
 }
 
 template <bool WP, typename PT, bool PIXAX>
-static cudaError_t gauss_launch_one(const NfLikeArgs &a, cudaStream_t st)
+static cudaError_t gauss_launch_one(const NfLikeArgs &a0, cudaStream_t st)
 {
     auto kern = nf_gauss_kernel<WP, PT, PIXAX>;
-    const size_t smem = 128 + (((size_t)a.n_pad * 4 + 127) / 128) * 128 + sizeof(GaussScratch) * NF_WARPS_PER_CTA;
+    NfLikeArgs a = a0;
+    // the tile's pixel is staged in shared memory by one bulk copy; rows too long for that are read from HBM / L2
+    a.stage = WP ? 0 : 1;
+    auto smem_bytes = [&] {
+        return 128 + (a.stage ? (((size_t)a.n_pad * 4 + 127) / 128) * 128 : 0) + sizeof(GaussScratch) * NF_WARPS_PER_CTA;
+    };
+    size_t smem = smem_bytes();
+    if (smem > 227 * 1024 && a.stage) {
+        a.stage = 0;
+        smem = smem_bytes();
+    }
     if (smem > 227 * 1024) return cudaErrorInvalidConfiguration;
     cudaError_t e = nf_ensure_dyn_smem((const void *)kern, smem);
     if (e) return e;

@@ -213,8 +213,12 @@ __device__ __noinline__ void nh3_setup_batch(const NfLikeArgs &a, SC &sc, int64_
     tau_main = pop * sm.fracterm * ((1.0 - e) / (1.0 + e)) * (sm.width_c / sigm);
     }
     // T_B amplitude T0_j * (G(T0_j/tex) - tbg_j), hyperfine.pyx:106-113, as the max of two
-    // lines in j: the reference's G is a convex piecewise-linear table, so this reproduces
-    // the table lerp -- including a knot inside the band -- without per-channel look-ups.
+    // lines in j: the reference's G is a convex piecewise-linear table, and the lines of the
+    // table segments at the two band edges reproduce it exactly while the band crosses at most
+    // one knot (about 1e-3 of nu); beyond, G is underestimated between the outer knots.  With
+    // tbg and T0 made linear in j the amplitude is within 6.2e-6 of its peak up to
+    // NF_MAX_BAND_FRAC over tex >= 2.8 K, error growing as the band squared (the pixel-block
+    // constructors refuse wider hyperfine spectra; tests/test_amplitude_model.py).
     const double nm1 = (double)(nh3_nchan_of<PIXAX>(a, pix, s) - 1);
     const double xL = sm.T0_first / tex, xR = sm.T0_last / tex;
     const double dxdj = (xR - xL) / nm1;
@@ -237,8 +241,8 @@ __device__ __noinline__ void nh3_setup_batch(const NfLikeArgs &a, SC &sc, int64_
         aL = aR = gL;
         bL = bR = (gR - gL) / nm1;
     }
-    // fold T0_j = T0_first + (T0_last - T0_first) j / (N-1) into both lines (the j^2 term
-    // of the product is below 1e-8 of the amplitude): line through the end-channel values
+    // fold T0_j = T0_first + (T0_last - T0_first) j / (N-1) into both lines through their
+    // end-channel values (the j^2 term of the product is dropped: it grows as the band squared)
     const double pL0 = sm.T0_first * (aL - sm.tbg0);
     const double pL1 = sm.T0_last * (aL + bL * nm1 - sm.tbg0 - sm.tbg1 * nm1);
     const double pR0 = sm.T0_first * (aR - sm.tbg0);

@@ -20,6 +20,17 @@ _MODELS = {"ammonia": _lib.NF_MODEL_NH3, "gaussian": _lib.NF_MODEL_GAUSS, "diaze
 _N_MODEL = {_lib.NF_MODEL_NH3: 6, _lib.NF_MODEL_N2HP: 4, _lib.NF_MODEL_GAUSS: 3}
 
 
+def _check_band(model, x):
+    """The hyperfine models' brightness amplitude is linear in the channel, which holds to the suite's accuracy up
+    to a fractional bandwidth of NF_MAX_BAND_FRAC (include/nestfit_b200.h)."""
+    if model != _lib.NF_MODEL_GAUSS:
+        frac = (x[-1] - x[0]) / x[0]
+        if not frac <= _lib.NF_MAX_BAND_FRAC:
+            raise ValueError(f"spectrum spans {frac:.4g} of its lowest frequency; the hyperfine models accept at most "
+                             f"NF_MAX_BAND_FRAC = {_lib.NF_MAX_BAND_FRAC:g} (about "
+                             f"{_lib.NF_MAX_BAND_FRAC * 299792.458:.0f} km/s)")
+
+
 class PixelBlock:
     per_pixel_axes = False
 
@@ -33,7 +44,6 @@ class PixelBlock:
         rest_freq : Gaussian-model rest frequency [Hz]
         """
         from .core import check_uniform_axis
-        lib = _lib.load()
         self.model_name = model
         self.model = _MODELS[model]
         xarrs = [np.ascontiguousarray(x, dtype=np.float64) for x in xarrs]
@@ -43,6 +53,8 @@ class PixelBlock:
             if x.shape[0] != self.n_chan:
                 raise ValueError("all spectra of a block must have the same number of channels")
             check_uniform_axis(x)
+            _check_band(self.model, x)
+        lib = _lib.load()
         self.xarrs = xarrs
         data = np.asarray(data)
         if data.dtype not in (np.float32, np.float64):
@@ -84,7 +96,6 @@ class PixelBlock:
         ``predict`` needs ``pix_of_vec`` and returns rows of ``n_chan_max`` channels, zero past each spectrum's end.
         """
         from .core import check_uniform_axis
-        lib = _lib.load()
         self = cls.__new__(cls)
         self.model_name = model
         self.model = _MODELS[model]
@@ -110,6 +121,7 @@ class PixelBlock:
             for k, s in enumerate(sp):
                 x = np.ascontiguousarray(s.xarr, dtype=np.float64)
                 check_uniform_axis(x)
+                _check_band(self.model, x)
                 d = np.asarray(s.data, dtype=np.float64)
                 if d.shape != x.shape:
                     raise ValueError(f"pixel {p} spectrum {k}: data and axis lengths differ")
@@ -129,6 +141,7 @@ class PixelBlock:
         self.trans_ids, self.rest_freq = tid, rf
         self.device = device
         self.n_model = _N_MODEL[self.model]
+        lib = _lib.load()
         out = C.c_void_p()
         _lib.check(lib.nf_pixels_create_axes(device, self.model, n_pix, n_spec, n_chan_max, _lib.ptr(nu_min),
                                              _lib.ptr(nu_chan), _lib.ptr(n_chan), _lib.ptr(tid), _lib.ptr(rf),

@@ -4,7 +4,10 @@ exponent), the same FP32 operation order in the pair term and the radiative-tran
 2^-5), with MUFU.EX2's relative error modelled as a random 2^-22 perturbation.  The FP64 set-up (partition function,
 main-line optical depth, brightness amplitude) is taken from the C oracle, so a comparison with the oracle's
 spectra isolates the error budget of the FP32 part -- a CPU test bed for changes to the record algebra before they
-cost GPU time.  Development tool and test infrastructure: nothing under nestfit_b200/ imports it.
+cost GPU time.  `amplitude` restates the set-up's brightness amplitude (nf_capi.cu fill_spec_meta, nf_nh3.cu
+nh3_setup_batch and the radiative-transfer step of phase M) on its own, so that its error can be compared with the
+oracle's per-channel T0_j (G(T0_j / tex) - tbg_j).  Development tool and test infrastructure: nothing under
+nestfit_b200/ imports it.
 
   python tools/kernel_model.py [n_vectors]     error statistics against the oracle for prior-drawn vectors
 """
@@ -36,6 +39,60 @@ def load_tables():
     return dict(nu=_macro(text, 'NF_NH3_REST_FREQ_INIT'), ea=_macro(text, 'NF_NH3_EINSTEIN_A_INIT'),
                 off=_macro(text, 'NF_NH3_LINE_OFFSET_INIT').astype(int), voff=_macro(text, 'NF_NH3_LINE_VOFF_INIT'),
                 wts=_macro(text, 'NF_NH3_LINE_WEIGHT_INIT'))
+
+
+# the 1/(e^x - 1) table of hyperfine.pyx:12-20 as nf_nh3.cu uploads it
+IEM_SIZE = 1000
+IEM_XMIN = H * 23.0e9 / KB / 8.0
+IEM_XMAX = H * 28.0e9 / KB / 2.7
+IEM_STEP = (IEM_XMAX - IEM_XMIN) / (IEM_SIZE - 1)
+IEM_INV_DX = 1.0 / ((IEM_XMIN + IEM_STEP) - IEM_XMIN)
+IEM_Y = 1.0 / (np.exp(np.append(IEM_XMIN + np.arange(IEM_SIZE - 1) * IEM_STEP, IEM_XMAX)) - 1.0)
+
+
+def _iemtex(x):
+    """nh3_iemtex: table lerp inside the table's domain, 1/expm1 outside."""
+    if IEM_XMIN < x < IEM_XMAX:
+        k = min(int((x - IEM_XMIN) * IEM_INV_DX), IEM_SIZE - 2)
+        return (IEM_Y[k + 1] - IEM_Y[k]) * IEM_INV_DX * (x - (IEM_XMIN + k * IEM_STEP)) + IEM_Y[k]
+    return 1.0 / np.expm1(x)
+
+
+def amplitude(nu_min, nu_chan, n, tex):
+    """The brightness amplitude T0_j (G(T0_j / tex) - tbg_j) of channels j = 0 .. n-1 of the axis
+    nu_min + j nu_chan the way the kernel evaluates it (float32 [n]): the set-up (FP64) makes tbg and T0 linear in j
+    and G the larger of two lines taken from the table segments at the two band edges; phase M evaluates both lines
+    with one FP32 FMA each and takes their maximum."""
+    # fill_spec_meta (nf_capi.cu)
+    T0_first = H * nu_min / KB
+    T0_last = H * (nu_min + (n - 1) * nu_chan) / KB
+    nm1 = float(n - 1)
+    tbg0 = 1.0 / np.expm1(T0_first / TCMB)
+    tbg1 = (1.0 / np.expm1(T0_last / TCMB) - tbg0) / nm1
+    # nh3_setup_batch (nf_nh3.cu)
+    xL, xR = T0_first / tex, T0_last / tex
+    dxdj = (xR - xL) / nm1
+    if IEM_XMIN < xL < IEM_XMAX and IEM_XMIN < xR < IEM_XMAX:
+        lines = []
+        for xe in (xL, xR):
+            k = min(int((xe - IEM_XMIN) * IEM_INV_DX), IEM_SIZE - 2)
+            sl = (IEM_Y[k + 1] - IEM_Y[k]) * IEM_INV_DX
+            lines.append((IEM_Y[k] + sl * (xL - (IEM_XMIN + k * IEM_STEP)), sl * dxdj))
+        (aL, bL), (aR, bR) = lines
+    else:
+        gL, gR = _iemtex(xL), _iemtex(xR)
+        aL = aR = gL
+        bL = bR = (gR - gL) / nm1
+    pL0 = T0_first * (aL - tbg0)
+    pL1 = T0_last * (aL + bL * nm1 - tbg0 - tbg1 * nm1)
+    pR0 = T0_first * (aR - tbg0)
+    pR1 = T0_last * (aR + bR * nm1 - tbg0 - tbg1 * nm1)
+    am = np.array([pL0, pR0, (pL1 - pL0) / nm1, (pR1 - pR0) / nm1]).astype(F32)
+    # phase M: fma2(slope, j, intercept) per line, then the larger of the two
+    j = np.arange(n, dtype=F32)
+    fL = (am[2].astype(np.float64) * j + am[0]).astype(F32)       # one rounding: an FMA
+    fR = (am[3].astype(np.float64) * j + am[1]).astype(F32)
+    return np.maximum(fL, fR)
 
 
 def _ex2(a, rng):
