@@ -153,6 +153,17 @@ int nf_gauss_predict(const nf_pixels *px, const void *params_dev, int param_dtyp
 int nf_predict_pix(const nf_pixels *px, const void *params_dev, int param_dtype,
                    const int32_t *pix_of_vec_dev, int64_t B, int ncomp, int flags,
                    float *pred_dev, void *stream);
+/* Moments of single-component model spectra (hyperfine models only; NF_EINVAL
+ * for the Gaussian model): `params_dev` [B][n_model] of `param_dtype`; vector b
+ * is synthesised exactly as the *_predict calls do, on the axes of pixel
+ * pix_of_vec_dev[b] (required on a block with per-pixel axes, may be NULL on a
+ * shared-axis block), and reduced over the spectrum's own channels to
+ * peak_dev [B][n_spec] FP32 = its maximum (K) and sum_dev [B][n_spec] FP64 =
+ * its sum (K channel, accumulated in FP64).  No model row is written.  `flags`
+ * as for NH3 (ignored by N2H+). */
+int nf_predict_moments(const nf_pixels *px, const void *params_dev, int param_dtype,
+                       const int32_t *pix_of_vec_dev, int64_t B, int flags,
+                       float *peak_dev, double *sum_dev, void *stream);
 
 /* ---- host-buffer entry points (the call a reference-side binding makes) -- */
 /* params_host [B][ndim] of param_dtype, pix_of_vec_host may be NULL (then
@@ -180,6 +191,9 @@ int nf_n2hp_predict_host(const nf_pixels *px, const void *params_host, int param
 int nf_predict_pix_host(const nf_pixels *px, const void *params_host, int param_dtype,
                         const int32_t *pix_of_vec_host, int64_t B, int ncomp, int flags,
                         float *pred_host);
+int nf_predict_moments_host(const nf_pixels *px, const void *params_host, int param_dtype,
+                            const int32_t *pix_of_vec_host, int64_t B, int flags,
+                            float *peak_host, double *sum_host);
 
 /* ---- prior transform ---------------------------------------------------- */
 int nf_priors_create(int device, const nf_prior_desc *priors, int n_prior,
@@ -252,6 +266,14 @@ int nf_ns_posterior(const nf_sampler *s, int64_t run, int32_t capacity, float *t
  *     interpolation, like Dumper.calc_marginals (core.pyx:596-598) -- sorted on the device.  Either may be NULL. */
 int nf_ns_products_rows(nf_sampler *s, int64_t *row_offsets);
 int nf_ns_products(nf_sampler *s, const double *quantiles, int n_q, float *post, double *marginals);
+/* Credible intervals of each component's peak and integrated intensity (hyperfine models; NF_EINVAL for the
+ * Gaussian model and before nf_ns_products_rows).  Every posterior row of every run (the rows
+ * nf_ns_products_rows counts) is split into its `ncomp` single-component vectors, which are synthesised on the
+ * run's pixel as nf_predict_moments does; then, per (run, spectrum, component), the posterior-weighted quantiles
+ * of the peak (K) and of the channel sum (K channel), with the float32 weights of the `posteriors` rows and the
+ * rule of numpy.interp(q, cumsum(w_sorted) / sum(w), x_sorted).  peak_q, integ_q: host
+ * [n_run][n_q][n_spec][ncomp] FP64; either may be NULL. */
+int nf_ns_intensity(nf_sampler *s, const double *quantiles, int n_q, double *peak_q, double *integ_q);
 int nf_ns_stats(const nf_sampler *s, int32_t *lock_iters, int64_t *launches);
 
 /* ---- kernel timing helper (bench / roofline) ---------------------------- */

@@ -21,6 +21,7 @@ from .main import (  # noqa: F401
 from . import postprocess  # noqa: F401
 from .postprocess import (  # noqa: F401
     take_by_components, apply_circular_mask, get_indep_info_kernel, aggregate_run_attributes, convolve_evidence,
-    extended_masked_evidence, aggregate_run_products, aggregate_run_pdfs, convolve_post_pdfs,
+    extended_masked_evidence, aggregate_run_products, aggregate_intensity_marginals, aggregate_run_pdfs,
+    convolve_post_pdfs,
     quantize_conv_marginals, deblend_hf_intensity, generate_predicted_profiles, postprocess_run,
 )

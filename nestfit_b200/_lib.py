@@ -73,6 +73,8 @@ _SIGNATURES = {
     "nf_gauss_predict_host": ([_VP, _VP, _I, _I64, _I, _VP], _I),
     "nf_predict_pix": ([_VP, _VP, _I, _VP, _I64, _I, _I, _VP, _VP], _I),
     "nf_predict_pix_host": ([_VP, _VP, _I, _VP, _I64, _I, _I, _VP], _I),
+    "nf_predict_moments": ([_VP, _VP, _I, _VP, _I64, _I, _VP, _VP, _VP], _I),
+    "nf_predict_moments_host": ([_VP, _VP, _I, _VP, _I64, _I, _VP, _VP], _I),
     "nf_priors_create": ([_I, _VP, _I, _VP, _I, _VP, _I64, _I, C.POINTER(_VP)], _I),
     "nf_priors_free": ([_VP], _I),
     "nf_prior_transform": ([_VP, _VP, _I64, _I, _VP], _I),

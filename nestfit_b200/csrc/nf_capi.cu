@@ -314,13 +314,16 @@ int run_device(const nf_pixels *px, const NfLikeArgs &a, void *stream)
 // reference-side caller hands over) would serialise the pipeline -- a device-to-host copy into pageable memory
 // returns only when the kernel before it has finished -- so the log-likelihood call bounces them through a
 // page-locked ring: the host copies chunk k+1 into the ring while the kernel of chunk k runs.
+// Moments (peak_host / sum_host, [B][n_spec]) take the place of lnL_host and bounce like it.
 int run_host(const nf_pixels *px, int model, const void *params_host, int param_dtype,
              const int32_t *pix_host, int64_t vecs_per_pix, int64_t B, int ncomp, int flags,
-             double *lnL_host, float *pred_host)
+             double *lnL_host, float *pred_host, float *peak_host = nullptr, double *sum_host = nullptr)
 {
     if (!px || px->model != model) return NF_EINVAL;
     if (B == 0) return NF_OK;
-    if (!params_host || (!lnL_host && !pred_host)) return NF_EINVAL;
+    const bool want_mom = peak_host != nullptr;
+    if (want_mom && (!sum_host || lnL_host || pred_host)) return NF_EINVAL;
+    if (!params_host || (!lnL_host && !pred_host && !want_mom)) return NF_EINVAL;
     DeviceGuard g(px->device);
     if (!g.ok) return NF_ENODEV;
     const int n_model = model_nparams(model);
@@ -338,14 +341,18 @@ int run_host(const nf_pixels *px, int model, const void *params_host, int param_
     if (chunk > B) chunk = B;
     const size_t off_pix = (((size_t)chunk * ndim * psz) + 255) / 256 * 256;
     const size_t off_lnl = off_pix + (((size_t)chunk * 4) + 255) / 256 * 256;
-    const size_t off_pred = off_lnl + (((size_t)chunk * 8) + 255) / 256 * 256;
+    const size_t mom_peak_per_vec = want_mom ? (size_t)px->n_spec * 4 : 0;
+    const size_t off_mpk = off_lnl + (((size_t)chunk * 8) + 255) / 256 * 256;
+    const size_t off_msum = off_mpk + (((size_t)chunk * mom_peak_per_vec) + 255) / 256 * 256;
+    const size_t off_pred = off_msum + (((size_t)chunk * 2 * mom_peak_per_vec) + 255) / 256 * 256;
     const size_t total = off_pred + (size_t)chunk * pred_per_vec;
     // the block's two streams and staging buffers serve one host-buffer call at a time
     std::lock_guard<std::mutex> host_lock(*px->host_mu);
     int rc = ensure_stage(px, total);
     if (rc != NF_OK) return rc;
     const bool bounce = !want_pred && (!host_ptr_is_pinned(params_host) || !host_ptr_is_pinned(pix_host) ||
-                                       !host_ptr_is_pinned(lnL_host));
+                                       !host_ptr_is_pinned(lnL_host) || !host_ptr_is_pinned(peak_host) ||
+                                       !host_ptr_is_pinned(sum_host));
     if (bounce && (rc = ensure_stage_host(px, off_pred)) != NF_OK) return rc;
 
     constexpr int S = NF_HOST_SLOTS;
@@ -363,6 +370,13 @@ int run_host(const nf_pixels *px, int model, const void *params_host, int param_
         if (bounce && lnL_host)
             std::memcpy(lnL_host + pend_b0[slot], (const unsigned char *)px->stage_host[slot] + off_lnl,
                         (size_t)pend_nb[slot] * 8);
+        if (bounce && want_mom) {
+            std::memcpy((unsigned char *)peak_host + (size_t)pend_b0[slot] * mom_peak_per_vec,
+                        (const unsigned char *)px->stage_host[slot] + off_mpk, (size_t)pend_nb[slot] * mom_peak_per_vec);
+            std::memcpy((unsigned char *)sum_host + (size_t)pend_b0[slot] * 2 * mom_peak_per_vec,
+                        (const unsigned char *)px->stage_host[slot] + off_msum,
+                        (size_t)pend_nb[slot] * 2 * mom_peak_per_vec);
+        }
         pending[slot] = false;
     };
     // errors inside the pipeline leave through `status` so that the events are always destroyed
@@ -403,6 +417,10 @@ int run_host(const nf_pixels *px, int model, const void *params_host, int param_
                        lnL_host ? (double *)(dev + off_lnl) : nullptr,
                        want_pred ? (float *)(dev + off_pred) : nullptr, lnL_host != nullptr, &a);
         if (rc != NF_OK) { status = rc; break; }
+        if (want_mom) {
+            a.mom_peak = (float *)(dev + off_mpk);
+            a.mom_sum = (double *)(dev + off_msum);
+        }
         if (!pix_host && lnL_host) {
             // implicit pixel map continues across chunks: shift by whole pixels
             a.data = px->data + (b0 / a.vecs_per_pix) * a.pix_stride;
@@ -423,6 +441,14 @@ int run_host(const nf_pixels *px, int model, const void *params_host, int param_
         if (want_pred)
             NF_STEP(cudaMemcpyAsync((unsigned char *)pred_host + (size_t)b0 * pred_per_vec, dev + off_pred,
                                     (size_t)nb * pred_per_vec, cudaMemcpyDeviceToHost, st));
+        if (want_mom) {
+            NF_STEP(cudaMemcpyAsync(bounce ? (void *)(ring + off_mpk)
+                                           : (void *)((unsigned char *)peak_host + (size_t)b0 * mom_peak_per_vec),
+                                    dev + off_mpk, (size_t)nb * mom_peak_per_vec, cudaMemcpyDeviceToHost, st));
+            NF_STEP(cudaMemcpyAsync(bounce ? (void *)(ring + off_msum)
+                                           : (void *)((unsigned char *)sum_host + (size_t)b0 * 2 * mom_peak_per_vec),
+                                    dev + off_msum, (size_t)nb * 2 * mom_peak_per_vec, cudaMemcpyDeviceToHost, st));
+        }
     }
 #undef NF_STEP
     // the chunks still in flight, oldest first
@@ -724,6 +750,28 @@ int nf_predict_pix_host(const nf_pixels *px, const void *params_host, int param_
 {
     if (!px || !pred_host || !pix_of_vec_host) return NF_EINVAL;
     return run_host(px, px->model, params_host, param_dtype, pix_of_vec_host, 1, B, ncomp, flags, nullptr, pred_host);
+}
+
+int nf_predict_moments(const nf_pixels *px, const void *params_dev, int param_dtype, const int32_t *pix_of_vec_dev,
+                       int64_t B, int flags, float *peak_dev, double *sum_dev, void *stream)
+{
+    if (!px || !is_hyperfine(px->model) || !peak_dev || !sum_dev || (px->pixmeta && !pix_of_vec_dev)) return NF_EINVAL;
+    NfLikeArgs a;
+    int rc = make_args(px, params_dev, param_dtype, pix_of_vec_dev, 1, B, 1, px->model == NF_MODEL_NH3 ? flags : 0,
+                       nullptr, nullptr, false, &a);
+    if (rc != NF_OK) return rc;
+    a.mom_peak = peak_dev;
+    a.mom_sum = sum_dev;
+    return run_device(px, a, stream);
+}
+
+int nf_predict_moments_host(const nf_pixels *px, const void *params_host, int param_dtype,
+                            const int32_t *pix_of_vec_host, int64_t B, int flags, float *peak_host, double *sum_host)
+{
+    if (!px || !is_hyperfine(px->model) || !peak_host || !sum_host || (px->pixmeta && !pix_of_vec_host))
+        return NF_EINVAL;
+    return run_host(px, px->model, params_host, param_dtype, pix_of_vec_host, 1, B, 1,
+                    px->model == NF_MODEL_NH3 ? flags : 0, nullptr, nullptr, peak_host, sum_host);
 }
 
 int nf_last_call_stats(double *kernel_ms, int64_t *n_launches)

@@ -105,6 +105,8 @@ struct NfLikeArgs {
     NfSpecMeta spec[NF_MAX_SPEC];
     const NfPixSpecMeta *pixmeta;   // per-pixel axes [n_pix][n_spec] (NULL: every pixel uses spec[]); n_chan is then the
                                     // longest spectrum and pred rows are that long
+    float *mom_peak;            // may be NULL: hyperfine kernel, ncomp 1, [B][n_spec] maximum of the model over the
+    double *mom_sum;            // spectrum's own channels, and its sum (replaces pred)
 };
 
 // launchers (nf_model.cu)

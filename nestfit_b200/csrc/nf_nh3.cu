@@ -347,7 +347,9 @@ __device__ __forceinline__ void blk_m_add(uint32_t ma, const float (&val)[8])
 
 // PIXAX: every pixel has its own axes and channel counts (a.pixmeta); a.n_chan is the longest spectrum, and the
 // super-blocks and the residual run to it (data and model are zero past a spectrum's own end).
-template <int MODEL, int NC, bool WRITE_PRED, typename PT, bool PIXAX>
+// MOM (with WRITE_PRED): instead of the model row, its maximum and its sum over the spectrum's own channels per
+// (vector, spectrum) -> a.mom_peak (FP32) and a.mom_sum (FP64, summed in FP64 per lane and across the warp).
+template <int MODEL, int NC, bool WRITE_PRED, typename PT, bool PIXAX, bool MOM = false>
 __global__ void __launch_bounds__(NF_THREADS, (NC <= 3 ? BLK_MINCTA : 2))
 nf_nh3_kernel(const __grid_constant__ NfLikeArgs a)
 {
@@ -477,6 +479,8 @@ nf_nh3_kernel(const __grid_constant__ NfLikeArgs a)
                 const char *grow = nullptr;
                 if (have_data) grow = reinterpret_cast<const char *>(a.data + pix * a.pix_stride + (int64_t)s * a.n_pad);
                 uint64_t acc_a = 0ull, acc_b = 0ull;        // packed FP32x2 sums of squared residuals
+                [[maybe_unused]] float mom_pk = -INFINITY;  // MOM: the lane's maximum and FP64 sum of the model
+                [[maybe_unused]] double mom_sum = 0.0;
                 for (int sbk = 0; sbk < n_sb; ++sbk) {
                     const int blk0 = sbk * BLK_SB;
                     // ---- T: items of the super-block, lanes <-> four consecutive blocks ----
@@ -651,12 +655,23 @@ nf_nh3_kernel(const __grid_constant__ NfLikeArgs a)
                     const int ch0 = blk0 << 3;
                     const int nch = min(BLK_SB * 8, a.n_pad - ch0);      // padded channels (data and model are zero there)
                     if (WRITE_PRED) {
+                        if constexpr (MOM) {
+                            // the channels WRITE_PRED writes, without those past the spectrum's end (0 there)
+                            const int nreal = min(BLK_SB * 8, (PIXAX ? n_own : a.n_chan) - ch0);
+                            for (int j = lane; j < nreal; j += 32) {
+                                const int bq = j >> 3;
+                                const float mv = sc.m[(blk_m_off(bq) + ((j >> 2) & 1) * BLK_PLANE) / 4 + (j & 3)];
+                                mom_pk = fmaxf(mom_pk, mv);
+                                mom_sum += (double)mv;
+                            }
+                        } else {
                         float *row = a.pred + (b * n_spec + s) * (int64_t)a.n_chan;
                         const int nreal = min(BLK_SB * 8, a.n_chan - ch0);
                         for (int j = lane; j < nreal; j += 32) {
                             const int bq = j >> 3;
                             const float mv = sc.m[(blk_m_off(bq) + ((j >> 2) & 1) * BLK_PLANE) / 4 + (j & 3)];
                             row[ch0 + j] = (PIXAX && ch0 + j >= n_own) ? 0.0f : mv;   // past the spectrum's end
+                        }
                         }
                         __syncwarp();
                         for (int idx = lane; idx < BLK_M_BYTES / 4; idx += 32) sc.m[idx] = 0.0f;
@@ -699,6 +714,15 @@ nf_nh3_kernel(const __grid_constant__ NfLikeArgs a)
                     const double tot = warp_sum((double)((a0 + a1) + (a2 + a3)));
                     lnl -= tot * __ldg(a.inv2s2 + pix * n_spec + s);
                 }
+                if constexpr (MOM) {
+#pragma unroll
+                    for (int o = 16; o > 0; o >>= 1) mom_pk = fmaxf(mom_pk, __shfl_xor_sync(NF_FULL, mom_pk, o));
+                    const double tot = warp_sum(mom_sum);
+                    if (lane == 0) {
+                        a.mom_peak[b * n_spec + s] = mom_pk;
+                        a.mom_sum[b * n_spec + s] = tot;
+                    }
+                }
                 __syncwarp();
             }
             if (a.lnL && lane == 0) a.lnL[b] = lnl;
@@ -716,7 +740,7 @@ static size_t nh3_smem_bytes(const NfLikeArgs &a, int nwarps)
     return 128 + data + ((size_t)NC * a.npair * 24 + (size_t)NC * a.nkey * sizeof(short2) + sizeof(BlkScratch<NC>)) * nwarps;
 }
 
-template <int MODEL, int NC, bool WP, typename PT, bool PIXAX>
+template <int MODEL, int NC, bool WP, typename PT, bool PIXAX, bool MOM = false>
 static cudaError_t nh3_launch_one(const NfLikeArgs &a0, cudaStream_t st)
 {
     NfLikeArgs a = a0;
@@ -724,7 +748,7 @@ static cudaError_t nh3_launch_one(const NfLikeArgs &a0, cudaStream_t st)
     for (int s = 0; s < a.n_spec; ++s) max_lines = a.spec[s].nlines > max_lines ? a.spec[s].nlines : max_lines;
     a.npair = (max_lines + 1) & ~1;                            // records per component (even: 16-byte aligned arrays)
     a.nkey = a.n_chan > BLK_SB * 8 ? ((max_lines + 3) & ~3) : 0;   // line keys are only re-read by later super-blocks
-    auto kern = nf_nh3_kernel<MODEL, NC, WP, PT, PIXAX>;
+    auto kern = nf_nh3_kernel<MODEL, NC, WP, PT, PIXAX, MOM>;
     // the tile's pixel is staged in shared memory by one bulk copy; rows too long for that are read from HBM / L2
     a.stage = WP ? 0 : 1;
     size_t smem = nh3_smem_bytes<NC>(a, NH3_WARPS);
@@ -745,6 +769,12 @@ static cudaError_t nh3_launch_one(const NfLikeArgs &a0, cudaStream_t st)
 template <int MODEL, int NC, bool PIXAX>
 static cudaError_t nh3_launch_ax(const NfLikeArgs &a, cudaStream_t st)
 {
+    if (a.mom_peak) {       // moments of single-component models only
+        if constexpr (NC == 1)
+            return a.param_f64 ? nh3_launch_one<MODEL, 1, true, double, PIXAX, true>(a, st)
+                               : nh3_launch_one<MODEL, 1, true, float, PIXAX, true>(a, st);
+        return cudaErrorInvalidValue;
+    }
     const bool wp = a.pred != nullptr;
     if (a.param_f64)
         return wp ? nh3_launch_one<MODEL, NC, true, double, PIXAX>(a, st)

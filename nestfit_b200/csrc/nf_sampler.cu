@@ -28,6 +28,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
+#include <algorithm>
 #include <cstring>
 #include <new>
 #include <vector>
@@ -65,6 +66,7 @@ struct nf_sampler {
     int32_t *keep_n;                   // [n_run] (device)
     int64_t *post_off;                 // [n_run + 1] (device)
     std::vector<int64_t> *h_post_off;
+    bool post_ready;                   // nf_ns_products_rows has set post_off
     double *lnZ, *H, *lmax;            // [n_run]
     int32_t *n_dead, *it, *done, *n_it_lock;
     int64_t *n_eval;
@@ -1103,6 +1105,134 @@ ns_marginals_kernel(const float *post, const int64_t *post_off, const int32_t *r
     }
 }
 
+// ---- intensity credible intervals (nf_ns_intensity) ------------------------------------------------
+// The kept rows of runs [r0, r0 + n_r) (the rows ns_pack_post_kernel writes, in the same order), each split into
+// its ncomp single-component vectors on the run's pixel: vec [(row * ncomp + c)][n_model] FP32, vpix likewise, and
+// the row's float32 posterior weight, computed as ns_pack_post_kernel does.  Rows are counted from the group's
+// first row.  One warp per run, ordered compaction.
+__global__ void __launch_bounds__(128)
+ns_int_gather_kernel(const float *dead_th, const double *dead_l, const double *dead_lw, const int64_t *dead_off,
+                     const int32_t *n_dead, const double *lnZ, const int64_t *post_off, const int32_t *pix_ids,
+                     int64_t r0, int64_t n_r, int d, int ncomp, float *vec, int32_t *vpix, float *wt)
+{
+    const int64_t e = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (e >= n_r) return;
+    const int64_t r = r0 + e;
+    const int64_t off = dead_off[r], row0 = post_off[r] - post_off[r0];
+    const int nd = n_dead[r], nm = d / ncomp;
+    const double z = lnZ[r];
+    const int32_t pix = pix_ids[r];
+    int at = 0;
+    for (int base = 0; base < nd; base += 32) {
+        const int p = base + lane;
+        const double l = p < nd ? dead_l[off + p] : -INFINITY;
+        const bool keep = l > -INFINITY;
+        const unsigned m = __ballot_sync(NS_FULL, keep);
+        if (keep) {
+            const int64_t row = row0 + at + __popc(m & ((1u << lane) - 1u));
+            const float *th = dead_th + (off + p) * d;
+            for (int c = 0; c < ncomp; ++c) {             // parameter-major, component-minor rows
+                float *v = vec + (row * ncomp + c) * nm;
+                for (int j = 0; j < nm; ++j) v[j] = th[j * ncomp + c];
+                vpix[row * ncomp + c] = pix;
+            }
+            wt[row] = (float)exp(l + dead_lw[off + p] - z);
+        }
+        at += __popc(m);
+    }
+}
+
+// Posterior-weighted quantiles of one (entry of run_list, spectrum, component, quantity) per CTA, quantity 0 the
+// peak and 1 the channel sum of the component's model.  The (value, row) keys of the run's rows are sorted by a
+// bitonic network in shared memory (or in `scratch` for runs with more rows than fit): equal values keep their row
+// order, as numpy.argsort(kind='stable') -- duplicate rows (a final live point equal to a dead one) make the
+// interpolation depend on it.  The weights then become their running FP64 sum in row order of the sorted list, summed
+// one after the other like numpy.cumsum, and every quantile q is numpy.interp(q, cw / cw[-1], x_sorted), branch for
+// branch.  Each entry is a double value and an 8-byte slot holding {float weight, int row} while sorting and the
+// running sum after.
+struct NsWRow {
+    float w;
+    int row;
+};
+__global__ void __launch_bounds__(512)
+ns_wquant_kernel(const float *peak, const double *sum, const float *wt, const int64_t *post_off, int64_t row_base,
+                 const int32_t *run_list, int n_list, int n_spec, int ncomp, const double *quant, int n_q,
+                 double *peak_q, double *integ_q, double *scratch, int scratch_stride)
+{
+    extern __shared__ double s_kw[];
+    const int item = blockIdx.x;
+    const int per = n_spec * ncomp * 2;
+    const int e = item / per, rest = item - e * per;
+    if (e >= n_list) return;
+    const int qty = rest & 1, sc = rest >> 1, s = sc / ncomp, c = sc - s * ncomp;
+    const int r = run_list[e];
+    const int64_t o = post_off[r] - row_base;
+    const int n = (int)(post_off[r + 1] - post_off[r]);
+    const int tid = threadIdx.x, nt = blockDim.x;
+    int np2 = 1;
+    while (np2 < n) np2 <<= 1;
+    double *key = scratch ? scratch + (int64_t)item * 2 * scratch_stride : s_kw;
+    double *cw = key + (scratch ? scratch_stride : np2);
+    NsWRow *slot = reinterpret_cast<NsWRow *>(cw);
+    for (int i = tid; i < np2; i += nt) {
+        const int64_t v = ((o + i) * ncomp + c) * n_spec + s;
+        key[i] = i < n ? (qty ? sum[v] : (double)peak[v]) : INFINITY;
+        slot[i] = NsWRow{i < n ? wt[o + i] : 0.0f, i};
+    }
+    __syncthreads();
+    for (int k = 2; k <= np2; k <<= 1)
+        for (int st = k >> 1; st > 0; st >>= 1) {
+            for (int t = tid; t < (np2 >> 1); t += nt) {
+                const int lo = ((t & ~(st - 1)) << 1) | (t & (st - 1)), hi = lo | st;
+                const double a = key[lo], b = key[hi];
+                const NsWRow sa = slot[lo], sb = slot[hi];
+                const bool up = (lo & k) == 0;
+                if ((a > b || (a == b && sa.row > sb.row)) == up) {
+                    key[lo] = b; key[hi] = a;
+                    slot[lo] = sb; slot[hi] = sa;
+                }
+            }
+            __syncthreads();
+        }
+    if (tid == 0) {             // numpy.cumsum: one addition after the other
+        double run = 0.0;
+        for (int i = 0; i < n; ++i) {
+            run += (double)slot[i].w;
+            cw[i] = run;
+        }
+    }
+    __syncthreads();
+    if (tid < n_q) {
+        double v = nan("");
+        if (n > 0) {
+            const double q = quant[tid], tot = cw[n - 1];
+            int lo = 0, hi = n;              // j = (number of i with cw_i / tot <= q) - 1
+            while (lo < hi) {
+                const int mid = (lo + hi) >> 1;
+                if (q >= cw[mid] / tot) lo = mid + 1;
+                else hi = mid;
+            }
+            const int j = lo - 1;
+            if (j < 0) v = key[0];
+            else if (j >= n - 1) v = key[n - 1];
+            else {
+                const double xj = cw[j] / tot, xj1 = cw[j + 1] / tot;
+                if (xj == q) v = key[j];
+                else {
+                    const double slope = (key[j + 1] - key[j]) / (xj1 - xj);
+                    v = slope * (q - xj) + key[j];
+                    if (isnan(v)) {
+                        v = slope * (q - xj1) + key[j + 1];
+                        if (isnan(v) && key[j] == key[j + 1]) v = key[j];
+                    }
+                }
+            }
+        }
+        (qty ? integ_q : peak_q)[(((int64_t)r * n_q + tid) * n_spec + s) * ncomp + c] = v;
+    }
+}
+
 #define NS_CUDA(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) return (int)e__; } while (0)
 
 int score(nf_sampler *s, double *params, const int32_t *pix, int64_t vpp, int64_t B, double *lnl,
@@ -1293,6 +1423,7 @@ int nf_ns_run(nf_sampler *s)
     int prev = -1;
     cudaGetDevice(&prev);
     if (cudaSetDevice(s->device) != cudaSuccess) return NF_ENODEV;
+    s->post_ready = false;             // the row offsets of nf_ns_products_rows describe the previous run
     const int d = s->ndim, NL = s->cfg.nlive_max, K = s->K;
     const int64_t R = s->n_run;
     cudaStream_t st = s->stream;
@@ -1524,6 +1655,7 @@ int nf_ns_products_rows(nf_sampler *s, int64_t *row_offsets)
         e = cudaMemcpyAsync(s->post_off, off.data(), ((size_t)R + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(s->stream);
     }
+    s->post_ready = e == cudaSuccess;
     s->launches += 1;
     if (prev >= 0) cudaSetDevice(prev);
     return (int)e;
@@ -1604,6 +1736,142 @@ int nf_ns_products(nf_sampler *s, const double *quantiles, int n_q, float *post,
     ns_scratch_free(d_q, st);
     ns_scratch_free(d_marg, st);
     ns_scratch_free(d_list, st);
+    cudaStreamSynchronize(st);
+    if (prev >= 0) cudaSetDevice(prev);
+    return (int)e;
+}
+
+int nf_ns_intensity(nf_sampler *s, const double *quantiles, int n_q, double *peak_q, double *integ_q)
+{
+    if (!s || !s->post_ready || n_q < 1 || n_q > 64 || !quantiles) return NF_EINVAL;
+    const nf_pixels *px = s->px;
+    if (px->model != NF_MODEL_NH3 && px->model != NF_MODEL_N2HP) return NF_EINVAL;
+    int prev = -1;
+    cudaGetDevice(&prev);
+    if (cudaSetDevice(s->device) != cudaSuccess) return NF_ENODEV;
+    const int64_t R = s->n_run;
+    const int d = s->ndim, ncomp = s->ncomp, nm = d / ncomp, n_spec = px->n_spec;
+    const std::vector<int64_t> &off = *s->h_post_off;
+    cudaStream_t st = s->stream;
+    // runs go through in groups of contiguous rows whose vectors fit the scratch (a run larger than that alone):
+    // 2^23 vectors, about 0.4 GB of scratch at ncomp x 6 parameters and two spectra
+    int64_t max_rows = 0;
+    for (int64_t r = 0; r < R; ++r) max_rows = std::max(max_rows, off[(size_t)r + 1] - off[(size_t)r]);
+    const int64_t cap_vec = std::max((int64_t)1 << 23, max_rows * ncomp);
+    const int64_t cap_rows = cap_vec / ncomp;
+    const size_t out_n = (size_t)R * n_q * n_spec * ncomp;
+    float *d_vec = nullptr, *d_peak = nullptr, *d_wt = nullptr;
+    double *d_sum = nullptr, *d_q = nullptr, *d_pq = nullptr, *d_iq = nullptr, *d_scratch = nullptr;
+    int32_t *d_vpix = nullptr, *d_list = nullptr;
+    cudaError_t e = cudaSuccess;
+    auto A = [&](cudaError_t x) { if (e == cudaSuccess) e = x; };
+    A(ns_scratch_alloc((void **)&d_vec, (size_t)cap_vec * nm * sizeof(float), st));
+    A(ns_scratch_alloc((void **)&d_vpix, (size_t)cap_vec * sizeof(int32_t), st));
+    A(ns_scratch_alloc((void **)&d_peak, (size_t)cap_vec * n_spec * sizeof(float), st));
+    A(ns_scratch_alloc((void **)&d_sum, (size_t)cap_vec * n_spec * sizeof(double), st));
+    A(ns_scratch_alloc((void **)&d_wt, (size_t)cap_rows * sizeof(float), st));
+    A(ns_scratch_alloc((void **)&d_q, (size_t)n_q * sizeof(double), st));
+    A(ns_scratch_alloc((void **)&d_pq, out_n * sizeof(double), st));
+    A(ns_scratch_alloc((void **)&d_iq, out_n * sizeof(double), st));
+    A(ns_scratch_alloc((void **)&d_list, (size_t)R * sizeof(int32_t), st));
+    A(cudaMemcpyAsync(d_q, quantiles, (size_t)n_q * sizeof(double), cudaMemcpyHostToDevice, st));
+    // moments of single-component vectors: the model kernel's moments mode, the block's axes and flags
+    NfLikeArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.inv2s2 = px->inv2s2; a.params = d_vec; a.pix_of_vec = d_vpix; a.vecs_per_pix = 1;
+    a.pix_stride = (int64_t)n_spec * px->n_pad; a.param_f64 = 0; a.ncomp = 1;
+    a.n_spec = n_spec; a.n_chan = px->n_chan; a.n_pad = px->n_pad;
+    a.cold = (s->flags & NF_FLAG_COLD) != 0; a.lte = (s->flags & NF_FLAG_LTE) != 0;
+    for (int k = 0; k < n_spec; ++k) a.spec[k] = px->spec[k];
+    a.pixmeta = px->pixmeta; a.mom_peak = d_peak; a.mom_sum = d_sum;
+    const int SMEM_ROWS = 8192;                    // 16-byte entries (value, {weight, row}): at most 128 KB of shared memory
+    static_assert(8192 <= (1 << 14), "size classes 0..14 cover the shared-memory runs");
+    const int per_run = n_spec * ncomp * 2;
+    // the run lists of every group, in one host array that outlives all the copies from it: group [r0, r1) uses
+    // entries [r0, r1) here and in d_list, so no group waits for the one before
+    std::vector<int32_t> h_list((size_t)R), big;
+    for (int64_t r0 = 0; e == cudaSuccess && r0 < R;) {
+        int64_t r1 = r0 + 1;
+        while (r1 < R && off[(size_t)r1 + 1] - off[(size_t)r0] <= cap_rows) ++r1;
+        const int64_t rows = off[(size_t)r1] - off[(size_t)r0], n_r = r1 - r0;
+        if (rows > 0) {
+            ns_int_gather_kernel<<<(unsigned)((n_r * 32 + 127) / 128), 128, 0, st>>>(
+                s->dead_th, s->dead_l, s->dead_lw, s->dead_off, s->n_dead, s->lnZ, s->post_off, s->pix_ids, r0, n_r, d,
+                ncomp, d_vec, d_vpix, d_wt);
+            A(cudaGetLastError());
+            a.B = rows * ncomp;
+            if (e == cudaSuccess) A(px->model == NF_MODEL_NH3 ? nf_launch_nh3(a, st) : nf_launch_n2hp(a, st));
+            s->launches += 2;
+        }
+        // runs that fit shared memory go through one launch per power-of-two size class, each with the shared
+        // memory of its class (a long run does not lower the occupancy of the short ones); the others are sorted in
+        // global scratch
+        big.clear();
+        std::vector<int32_t> cls_n(15, 0);              // runs per class, class k: np2 = 2^k <= SMEM_ROWS
+        std::vector<int> run_cls((size_t)(r1 - r0), -1);
+        int big_np2 = 1;
+        for (int64_t r = r0; r < r1; ++r) {
+            const int64_t n = off[(size_t)r + 1] - off[(size_t)r];
+            int k = 0;
+            while ((int64_t)1 << k < n) ++k;
+            if (n <= SMEM_ROWS) { run_cls[(size_t)(r - r0)] = k; ++cls_n[(size_t)k]; }
+            else { big.push_back((int32_t)r); big_np2 = std::max(big_np2, 1 << k); }
+        }
+        std::vector<int32_t> cls_off(16, 0);
+        for (int k = 0; k < 15; ++k) cls_off[(size_t)k + 1] = cls_off[(size_t)k] + cls_n[(size_t)k];
+        int32_t *small = h_list.data() + r0, *d_small = d_list + r0;
+        const int32_t n_small = cls_off[15];
+        {
+            std::vector<int32_t> at(cls_off.begin(), cls_off.end() - 1);
+            for (int64_t r = r0; r < r1; ++r) {
+                const int k = run_cls[(size_t)(r - r0)];
+                if (k >= 0) small[at[(size_t)k]++] = (int32_t)r;
+            }
+        }
+        if (e == cudaSuccess && n_small > 0) {
+            A(cudaMemcpyAsync(d_small, small, (size_t)n_small * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+            for (int k = 0; k < 15 && e == cudaSuccess; ++k) {
+                const int nk = cls_n[(size_t)k];
+                if (nk == 0) continue;
+                const size_t smem = ((size_t)1 << k) * 2 * sizeof(double);
+                A(nf_ensure_dyn_smem((const void *)ns_wquant_kernel, smem));
+                if (e == cudaSuccess)
+                    ns_wquant_kernel<<<(unsigned)((int64_t)nk * per_run), 512, smem, st>>>(
+                        d_peak, d_sum, d_wt, s->post_off, off[(size_t)r0], d_small + cls_off[(size_t)k], nk, n_spec,
+                        ncomp, d_q, n_q, d_pq, d_iq, nullptr, 0);
+                A(cudaGetLastError());
+                s->launches += 1;
+            }
+        }
+        // bounded scratch: the long runs go through in batches
+        for (size_t b0 = 0; e == cudaSuccess && b0 < big.size();) {
+            const size_t per = (size_t)big_np2 * 2 * sizeof(double) * per_run;
+            size_t nb = (size_t)(1ull << 31) / per;
+            if (nb < 1) nb = 1;
+            if (nb > big.size() - b0) nb = big.size() - b0;
+            A(ns_scratch_alloc((void **)&d_scratch, nb * per, st));
+            std::copy(big.begin() + b0, big.begin() + b0 + nb, h_list.begin() + r0 + n_small + b0);
+            A(cudaMemcpyAsync(d_small + n_small + b0, small + n_small + b0, nb * sizeof(int32_t),
+                              cudaMemcpyHostToDevice, st));
+            if (e == cudaSuccess)
+                ns_wquant_kernel<<<(unsigned)(nb * per_run), 512, 0, st>>>(
+                    d_peak, d_sum, d_wt, s->post_off, off[(size_t)r0], d_small + n_small + b0, (int)nb, n_spec, ncomp,
+                    d_q, n_q, d_pq, d_iq, d_scratch, big_np2);
+            A(cudaGetLastError());
+            A(cudaStreamSynchronize(st));
+            ns_scratch_free(d_scratch, st);
+            d_scratch = nullptr;
+            s->launches += 1;
+            b0 += nb;
+        }
+        r0 = r1;
+    }
+    if (peak_q) A(cudaMemcpyAsync(peak_q, d_pq, out_n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (integ_q) A(cudaMemcpyAsync(integ_q, d_iq, out_n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    A(cudaStreamSynchronize(st));
+    for (void *p : {(void *)d_vec, (void *)d_vpix, (void *)d_peak, (void *)d_sum, (void *)d_wt, (void *)d_q,
+                    (void *)d_pq, (void *)d_iq, (void *)d_list})
+        ns_scratch_free(p, st);
     cudaStreamSynchronize(st);
     if (prev >= 0) cudaSetDevice(prev);
     return (int)e;

@@ -188,11 +188,12 @@ class _WaveWriter:
     """Background thread that turns finished samplers into store waves: the device pass over the posterior
     products, the one device-to-host copy and the file write of wave N overlap the sampling of wave N + 1."""
 
-    def __init__(self, sink, store_posteriors):
-        self.sink, self.store_posteriors = sink, store_posteriors
+    def __init__(self, sink, store_posteriors, intensity=False):
+        self.sink, self.store_posteriors, self.intensity = sink, store_posteriors, intensity
         self.q = _queue.Queue(maxsize=1)          # at most one finished sampler waits with its device pool
         self.error = None
         self.seconds = 0.0
+        self.intensity_seconds = 0.0
         self.rows = 0
         self.thread = threading.Thread(target=self._loop, daemon=True)
         self.thread.start()
@@ -206,7 +207,9 @@ class _WaveWriter:
             try:
                 if self.error is None:
                     t0 = time.perf_counter()
-                    self.sink.add_wave(make_wave(ns, sel, self.store_posteriors, **meta))
+                    wave = make_wave(ns, sel, self.store_posteriors, intensity=self.intensity, **meta)
+                    self.intensity_seconds += wave.intensity_seconds
+                    self.sink.add_wave(wave)
                     self.seconds += time.perf_counter() - t0
             except BaseException as exc:          # surfaces in the fitting thread at the next submit / close
                 self.error = exc
@@ -226,10 +229,14 @@ class _WaveWriter:
             raise self.error
 
 
-def make_wave(ns, sel, store_posteriors, i_lon, i_lat, null_lnZ, n_chan_tot):
-    """The runs `sel` (None = all) of a finished sampler as a store `Wave`."""
+def make_wave(ns, sel, store_posteriors, i_lon, i_lat, null_lnZ, n_chan_tot, intensity=False):
+    """The runs `sel` (None = all) of a finished sampler as a store `Wave`; with `intensity` it carries the runs'
+    intensity credible intervals (NestedSamplingBatch.intensity_marginals), computed before the sampler closes."""
     res = ns.results
     prod = ns.products_all(marginals=True, posteriors=store_posteriors)
+    t_i = time.perf_counter()
+    inten = ns.intensity_marginals() if intensity else None
+    t_i = time.perf_counter() - t_i
     off = prod['row_offsets']
     n_samples = np.diff(off)
     cols = run_attr_columns(ns.ndim, n_chan_tot, ns.nlive, null_lnZ, res, n_samples)
@@ -242,7 +249,11 @@ def make_wave(ns, sel, store_posteriors, i_lon, i_lat, null_lnZ, n_chan_tot):
         off = np.concatenate([[0], np.cumsum(n_samples[sel])])
         marg, best, mapf = marg[sel], best[sel], mapf[sel]
         i_lon, i_lat = np.asarray(i_lon)[sel], np.asarray(i_lat)[sel]
-    return Wave(ns.ncomp, ns.ndim, n_chan_tot, i_lon, i_lat, cols, off, post, marg, best, mapf)
+        if inten is not None:
+            inten = {k: v[sel] for k, v in inten.items()}
+    wave = Wave(ns.ncomp, ns.ndim, n_chan_tot, i_lon, i_lat, cols, off, post, marg, best, mapf, inten)
+    wave.intensity_seconds = t_i if intensity else 0.0
+    return wave
 
 
 class CubeFitter:
@@ -255,7 +266,8 @@ class CubeFitter:
 
     def __init__(self, stack, utrans, runner_cls, runner_kwargs=None, lnZ_thresh=11, ncomp_max=2, mn_kwargs=None,
                  nlive_snr_fact=5, n_prop=32, max_pixels_per_wave=16384, seed=1234, store_posteriors=True,
-                 n_streams=1, pixels_per_stream=1024, retry_margin=None, retry_chi2_sigma=6.0):
+                 n_streams=1, pixels_per_stream=1024, retry_margin=None, retry_chi2_sigma=6.0,
+                 intensity_marginals=False):
         """Same arguments as the reference (main.py:388-421) plus the batching knobs
         `n_prop` (proposals per pixel per lock-step iteration), `max_pixels_per_wave`
         (pixels in flight per device wave), `n_streams` (host threads / CUDA streams that
@@ -266,7 +278,11 @@ class CubeFitter:
         that fails the evidence threshold while its best chi-square is more than `retry_chi2_sigma` sigma
         above the channel count.  The repeats are a small extra wave per ncomp (~1-2 s of latency each).
         Sampler options ride in `mn_kwargs`: 'walks', 'method', 'max_samples_per_live' (rows of the posterior pool
-        per live point, default 64; runs that fill their share are repeated with four times as many)."""
+        per live point, default 64; runs that fill their share are repeated with four times as many).
+        `intensity_marginals` (NH3 / N2H+): every run written to the store also carries the posterior-weighted
+        quantiles of each component's peak and integrated intensity ('peak_intensity_marginals',
+        'integrated_intensity_marginals', (M, n_spec, ncomp)), computed on the device by the store writer before the
+        run's posterior leaves it; `aggregate_intensity_marginals` gathers them into maps."""
         self.stack = stack
         self.utrans = utrans
         self.runner_cls = runner_cls
@@ -285,6 +301,7 @@ class CubeFitter:
         self.retry_chi2_sigma = retry_chi2_sigma
         self.seed = seed
         self.store_posteriors = store_posteriors
+        self.intensity_marginals = intensity_marginals
         self.stats = {}
 
     def __getstate__(self):
@@ -320,12 +337,14 @@ class CubeFitter:
         all_lon, all_lat = (np.asarray(a) for a in indices)
         n_tot = all_lon.size
         model = self._model_name()
+        if self.intensity_marginals and model not in ('ammonia', 'diazenylium'):
+            raise ValueError("intensity_marginals: the Gaussian model's peak and area are its own parameters")
         sink = None
         if group_root is not None:
             sink = group_root if hasattr(group_root, 'add_wave') else GroupSink(group_root, self.store_posteriors)
             if hasattr(sink, 'store_posteriors'):
                 sink.store_posteriors = self.store_posteriors
-        writer = _WaveWriter(sink, self.store_posteriors) if sink is not None else None
+        writer = _WaveWriter(sink, self.store_posteriors, self.intensity_marginals) if sink is not None else None
         n_evals = 0
         out = dict(i_lon=all_lon, i_lat=all_lat, nbest=np.full(n_tot, -1, dtype=np.int32),
                    lnZ=nans((n_tot, self.ncomp_max + 1)), lnZ_err=nans((n_tot, self.ncomp_max + 1)),
@@ -478,7 +497,8 @@ class CubeFitter:
                     # time the writer worked (mostly hidden behind the next wave) and time the fit waited for it
                     out['store_seconds'] = out.get('store_seconds', 0.0) + writer.seconds
                     out['store_wait_seconds'] = out.get('store_wait_seconds', 0.0) + time.perf_counter() - t_w
-                    writer = _WaveWriter(sink, self.store_posteriors)
+                    out['intensity_seconds'] = out.get('intensity_seconds', 0.0) + writer.intensity_seconds
+                    writer = _WaveWriter(sink, self.store_posteriors, self.intensity_marginals)
                 blk.close()
         except BaseException:
             if writer is not None:
@@ -700,7 +720,8 @@ class CubeFitter:
 
 def _block_summary(res, block, worker):
     """What a worker reports back per block: scalars only (the per-pixel arrays are in the store)."""
-    keep = ('seconds', 'n_evals', 'n_retried', 'n_rescued', 'n_truncated', 'store_seconds', 'store_wait_seconds')
+    keep = ('seconds', 'n_evals', 'n_retried', 'n_rescued', 'n_truncated', 'store_seconds', 'store_wait_seconds',
+            'intensity_seconds')
     out = {k: res[k] for k in keep if k in res}
     out.update(block=block, worker=worker, n_pix=int(np.asarray(res.get('nbest', ())).size))
     for k in ('evals_by_ncomp', 'seconds_by_ncomp'):

@@ -15,6 +15,13 @@ import numpy as np
 
 from . import _lib
 
+C_KMS = 299792.458
+
+
+def channel_kms(x):
+    """Channel width of the ascending uniform axis x [Hz] in km/s, |dnu| / mean(nu) * c (DataCube.dv)."""
+    return abs(x[1] - x[0]) / x.mean() * C_KMS
+
 
 _MODELS = {"ammonia": _lib.NF_MODEL_NH3, "gaussian": _lib.NF_MODEL_GAUSS, "diazenylium": _lib.NF_MODEL_N2HP}
 _N_MODEL = {_lib.NF_MODEL_NH3: 6, _lib.NF_MODEL_N2HP: 4, _lib.NF_MODEL_GAUSS: 3}
@@ -76,6 +83,7 @@ class PixelBlock:
         else:
             rf = np.ascontiguousarray(np.broadcast_to(np.asarray(rest_freq, dtype=np.float64), (self.n_spec,)))
         self.trans_ids, self.rest_freq = tid, rf
+        self.chan_kms = np.array([channel_kms(x) for x in xarrs])           # [n_spec]
         self.device = device
         out = C.c_void_p()
         dtype = _lib.NF_F64 if data.dtype == np.float64 else _lib.NF_F32
@@ -116,6 +124,7 @@ class PixelBlock:
         nu_min = np.empty((n_pix, n_spec))
         nu_chan = np.empty((n_pix, n_spec))
         noise = np.empty((n_pix, n_spec))
+        chan_kms = np.empty((n_pix, n_spec))
         data = np.zeros((n_pix, n_spec, n_chan_max))
         for p, sp in enumerate(spectra):
             for k, s in enumerate(sp):
@@ -126,6 +135,7 @@ class PixelBlock:
                 if d.shape != x.shape:
                     raise ValueError(f"pixel {p} spectrum {k}: data and axis lengths differ")
                 nu_min[p, k], nu_chan[p, k] = x[0], x[1] - x[0]
+                chan_kms[p, k] = channel_kms(x)
                 noise[p, k] = s.noise
                 data[p, k, :x.shape[0]] = d
         tid = rf = None
@@ -138,6 +148,7 @@ class PixelBlock:
         self.n_pix, self.n_spec = n_pix, n_spec
         self.n_chan, self.n_chan_max = n_chan, n_chan_max
         self.xarrs = None
+        self.chan_kms = chan_kms                                            # [n_pix, n_spec]
         self.trans_ids, self.rest_freq = tid, rf
         self.device = device
         self.n_model = _N_MODEL[self.model]
@@ -243,6 +254,33 @@ class PixelBlock:
             rc = lib.nf_gauss_predict_host(self.handle, _lib.ptr(params), dt, B, ncomp, _lib.ptr(out))
         _lib.check(rc, "predict")
         return out
+
+    def moments(self, params, cold=False, lte=False, pix_of_vec=None):
+        """Peak and channel sum of single-component model spectra (NH3 and N2H+ blocks): params [B, n_model] ->
+        (peak float32 [B, n_spec] in K, sum float64 [B, n_spec] in K channel), each over the spectrum's own
+        channels.  The spectra are those ``predict`` synthesises; only their maximum and FP64 sum leave the device.
+        ``pix_of_vec`` as for ``predict`` (required on a block from ``from_spectra``)."""
+        if self.model == _lib.NF_MODEL_GAUSS:
+            raise ValueError("moments: the Gaussian model's peak and area are its own parameters")
+        params, dt = self._params(params)
+        if params.ndim != 2 or params.shape[1] != self.n_model:
+            raise ValueError(f"moments takes single-component vectors [B, {self.n_model}], got {params.shape}")
+        B = params.shape[0]
+        pv = None
+        if pix_of_vec is not None:
+            pv = np.ascontiguousarray(pix_of_vec, dtype=np.int32)
+            if pv.shape != (B,):
+                raise ValueError("pix_of_vec must have one entry per vector")
+            if B and (pv.min() < 0 or pv.max() >= self.n_pix):
+                raise ValueError("pix_of_vec out of range")
+        elif self.per_pixel_axes:
+            raise ValueError("a block with per-pixel axes needs pix_of_vec for moments")
+        flags = (_lib.NF_FLAG_COLD if cold else 0) | (_lib.NF_FLAG_LTE if lte else 0)
+        peak = np.empty((B, self.n_spec), dtype=np.float32)
+        total = np.empty((B, self.n_spec), dtype=np.float64)
+        _lib.check(_lib.load().nf_predict_moments_host(self.handle, _lib.ptr(params), dt, _lib.ptr(pv), B, flags,
+                                                        _lib.ptr(peak), _lib.ptr(total)), "moments")
+        return peak, total
 
     def last_call_stats(self):
         ms = C.c_double()

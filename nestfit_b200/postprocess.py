@@ -294,6 +294,36 @@ def aggregate_run_products(store):
     store.create_dataset('nbest_marginals', pardata.transpose(), group=dpath)
 
 
+def aggregate_intensity_marginals(store):
+    """'nbest_peak_intensity_marginals' (K) and 'nbest_integrated_intensity_marginals' (K km/s), (t, m, M, b, l):
+    the credible intervals of each component's peak and integrated intensity of the preferred model, gathered from
+    the runs of a fit made with intensity_marginals=True.  Uses 'conv_nbest' when the evidence was convolved, else
+    the per-pixel 'nbest', as aggregate_run_products does; positions and components without a run are NaN."""
+    from .store import INTENSITY_DATASETS
+    hdf, dpath = store.hdf, store.dpath
+    n_lon, n_lat = int(hdf.attrs['naxis1']), int(hdf.attrs['naxis2'])
+    key = 'conv_nbest' if f'{dpath}/conv_nbest' in hdf else 'nbest'
+    nbest_data = np.asarray(hdf[f'{dpath}/{key}'][...]).transpose()
+    ncomp_max = int(hdf.attrs['n_max_components'])
+    first = store.find_first_valid_group()
+    if INTENSITY_DATASETS[0] not in first:
+        raise ValueError('the runs of this store carry no intensity marginals: fit with intensity_marginals=True')
+    n_margs, n_spec = np.asarray(first[INTENSITY_DATASETS[0]][...]).shape[:2]
+    out = {name: nans((n_lon, n_lat, n_margs, ncomp_max, n_spec)) for name in INTENSITY_DATASETS}
+    for group in store.iter_pix_groups():
+        i_lon, i_lat = int(group.attrs['i_lon']), int(group.attrs['i_lat'])
+        nbest = int(nbest_data[i_lon, i_lat])
+        if nbest <= 0 or f'{nbest}' not in group:
+            continue
+        nb_group = group[f'{nbest}']
+        for name in INTENSITY_DATASETS:
+            if name not in nb_group:
+                raise ValueError(f'run /pix/{i_lon}/{i_lat}/{nbest} carries no {name}')
+            out[name][i_lon, i_lat, :, :nbest, :] = np.asarray(nb_group[name][...]).transpose(0, 2, 1)
+    for name, arr in out.items():
+        store.create_dataset(f'nbest_{name}', arr.transpose(), group=dpath)
+
+
 def aggregate_run_pdfs(store, par_bins=None):
     """'pdf_bins' (p, h) and 'post_pdfs' (r, m, p, h, b, l) (main.py:885-953)."""
     hdf, dpath = store.hdf, store.dpath

@@ -22,6 +22,7 @@ _lib.register("nf_ns_posterior", [_VP, _I64, C.c_int32, _VP, _VP, _VP])
 _lib.register("nf_ns_stats", [_VP, C.POINTER(C.c_int32), C.POINTER(_I64)])
 _lib.register("nf_ns_products_rows", [_VP, _VP])
 _lib.register("nf_ns_products", [_VP, _VP, _I, _VP, _VP])
+_lib.register("nf_ns_intensity", [_VP, _VP, _I, _VP, _VP])
 
 from .store import MARG_COLS, MARG_QUANTILES, run_attr_columns  # noqa: E402  (names re-exported)
 
@@ -122,6 +123,31 @@ class NestedSamplingBatch:
         self._batch = dict(row_offsets=off, posteriors=post, marginals=marg)
         return self._batch
 
+    def intensity_marginals(self, quantiles=MARG_QUANTILES):
+        """Posterior-weighted credible intervals of every component's peak and integrated intensity, computed on
+        the device from the run's posterior rows (NH3 and N2H+).  Returns {'peak_intensity_marginals' (K),
+        'integrated_intensity_marginals' (K km/s)}, each [n_run, len(quantiles), n_spec, ncomp].  The integrated
+        intensity is the model's channel sum times the channel width of the run's spectrum in km/s
+        (|dnu| / mean(nu) * c, as DataCube.dv)."""
+        if self.block.model == _lib.NF_MODEL_GAUSS:
+            raise ValueError("intensity_marginals: the Gaussian model's peak and area are its own parameters")
+        q = np.ascontiguousarray(quantiles, dtype=np.float64)
+        if q.ndim != 1 or not 1 <= q.size <= 64:
+            raise ValueError("intensity_marginals takes 1 to 64 quantiles")
+        self.results
+        lib = _lib.load()
+        if getattr(self, "_batch", None) is None:       # the rows of every run (nf_ns_products_rows)
+            off = np.empty(self.n_run + 1, dtype=np.int64)
+            _lib.check(lib.nf_ns_products_rows(self.handle, _lib.ptr(off)), "nf_ns_products_rows")
+        shape = (self.n_run, q.size, self.block.n_spec, self.ncomp)
+        peak, integ = np.empty(shape), np.empty(shape)
+        _lib.check(lib.nf_ns_intensity(self.handle, _lib.ptr(q), q.size, _lib.ptr(peak), _lib.ptr(integ)),
+                   "nf_ns_intensity")
+        kms = np.asarray(self.block.chan_kms, dtype=np.float64)
+        kms = kms[self.pix_ids] if kms.ndim == 2 else np.broadcast_to(kms, (self.n_run, kms.size))
+        integ *= kms[:, None, :, None]
+        return {'peak_intensity_marginals': peak, 'integrated_intensity_marginals': integ}
+
     @property
     def results(self):
         if self._results is None:
@@ -218,12 +244,17 @@ class Dumper:
 
 def run_multinest(runner, dumper, IS=False, mmodal=True, ceff=False, nlive=400, tol=0.5, efr=0.3, nClsPar=None,
                   maxModes=100, updInt=10, Ztol=-1e90, root='results', seed=-1, pWrap=None, fb=False,
-                  resume=False, initMPI=False, outfile=False, logZero=-1e100, maxiter=int(1e6), n_prop=32):
+                  resume=False, initMPI=False, outfile=False, logZero=-1e100, maxiter=int(1e6), n_prop=32,
+                  intensity_marginals=False):
     """Drop-in for the reference's ``run_multinest`` (core.pyx:727-823): fits the
     runner's pixel with the batched device sampler (one run), sets
     ``runner.run_lnZ`` and writes the reference's products through ``dumper``.
     MultiNest-only switches (IS, mmodal, ceff, nClsPar, maxModes, updInt, Ztol,
-    pWrap, fb, resume, initMPI, outfile, logZero, root) are accepted and ignored."""
+    pWrap, fb, resume, initMPI, outfile, logZero, root) are accepted and ignored.
+    With ``intensity_marginals`` the dumper also receives 'peak_intensity_marginals' and
+    'integrated_intensity_marginals' [15, n_spec, ncomp] (``NestedSamplingBatch.intensity_marginals``)."""
+    if intensity_marginals and runner._block.model == _lib.NF_MODEL_GAUSS:
+        raise ValueError("intensity_marginals: the Gaussian model's peak and area are its own parameters")
     assert runner.ndim > 0
     assert nlive > 0
     assert tol > 0
@@ -242,6 +273,8 @@ def run_multinest(runner, dumper, IS=False, mmodal=True, ceff=False, nlive=400, 
     runner.run_lnZ = float(res["lnZ"][0])
     if dumper is not None and not dumper.no_dump:
         attrs, dsets = ns.products(0, runner.null_lnZ, runner.n_chan_tot)
+        if intensity_marginals:
+            dsets.update({k: v[0] for k, v in ns.intensity_marginals().items()})
         dumper.append_attributes(**attrs)
         dumper.append_datasets(**dsets)
     dumper_calls = getattr(dumper, "n_calls", 0)
@@ -258,13 +291,15 @@ def _runner_spectra(runner):
     return [runner.spectrum] if spectra is None else list(spectra)
 
 
-def _check_batch(runners, dumpers, nlive, tol, efr, maxiter, max_runs_per_batch, nClsPar):
+def _check_batch(runners, dumpers, nlive, tol, efr, maxiter, max_runs_per_batch, nClsPar, intensity=False):
     """Argument checks of run_multinest_batch; touch no device."""
     if len(runners) == 0:
         raise ValueError("run_multinest_batch needs at least one runner")
     r0 = runners[0]
     if getattr(r0, "model_name", None) is None:
         raise ValueError(f"{type(r0).__name__} is not a runner of this package")
+    if intensity and r0.model_name == "gaussian":
+        raise ValueError("intensity_marginals: the Gaussian model's peak and area are its own parameters")
 
     def trans(r):
         return tuple(int(s.trans_id) for s in _runner_spectra(r))
@@ -299,7 +334,7 @@ def _check_batch(runners, dumpers, nlive, tol, efr, maxiter, max_runs_per_batch,
 
 
 def run_multinest_batch(runners, dumpers=None, nlive=400, tol=0.5, efr=0.3, seed=-1, maxiter=int(1e6), n_prop=32,
-                        max_runs_per_batch=16384, **multinest_switches):
+                        max_runs_per_batch=16384, intensity_marginals=False, **multinest_switches):
     """Batched form of ``run_multinest``: fits every runner's pixel in lock-step on the device.
 
     The runners may come from anywhere -- a catalogue of pointed observations, spectra cut from several cubes --
@@ -313,7 +348,9 @@ def run_multinest_batch(runners, dumpers=None, nlive=400, tol=0.5, efr=0.3, seed
     ``nlive`` is a scalar or one value per runner.  Truncated runs are flagged (``truncated``) but not repeated.
     MultiNest-only switches are accepted and ignored, as in ``run_multinest``.  Returns the per-runner result
     arrays (``lnZ``, ``lnZ_err``, ``max_loglike``, ``n_samples``, ``n_iter``, ``n_evals``, ``bestfit``,
-    ``mapfit``, ``truncated``) in runner order.
+    ``mapfit``, ``truncated``) in runner order.  With ``intensity_marginals`` every dumper also receives
+    'peak_intensity_marginals' and 'integrated_intensity_marginals' [15, n_spec, ncomp] of its run, computed on the
+    device from the batch's posteriors and scaled by that runner's own channel widths.
 
     Choosing the number of components stays the caller's loop, as with the reference: one call per ncomp over
     the sources that are still improving::
@@ -335,7 +372,8 @@ def run_multinest_batch(runners, dumpers=None, nlive=400, tol=0.5, efr=0.3, seed
     """
     from .pixels import PixelBlock
     runners = list(runners)
-    _check_batch(runners, dumpers, nlive, tol, efr, maxiter, max_runs_per_batch, multinest_switches.get("nClsPar"))
+    _check_batch(runners, dumpers, nlive, tol, efr, maxiter, max_runs_per_batch, multinest_switches.get("nClsPar"),
+                 intensity_marginals)
     n = len(runners)
     r0 = runners[0]
     dumpers = [None] * n if dumpers is None else list(dumpers)
@@ -355,6 +393,7 @@ def run_multinest_batch(runners, dumpers=None, nlive=400, tol=0.5, efr=0.3, seed
                 if any(dump):          # the posteriors of the whole batch in one device pass and one copy
                     prod = ns.products_all(marginals=False, posteriors=True)
                     off, pool = prod["row_offsets"], prod["posteriors"]
+                    inten = ns.intensity_marginals() if intensity_marginals else None
                 for j, i in enumerate(sel):
                     runner, dumper = runners[i], dumpers[i]
                     runner.run_lnZ = float(res["lnZ"][j])
@@ -365,6 +404,8 @@ def run_multinest_batch(runners, dumpers=None, nlive=400, tol=0.5, efr=0.3, seed
                             res["lnZ"][j], res["lnZ_err"][j], res["max_loglike"][j], res["bestfit"][j],
                             res["mapfit"][j], n_iter=res["n_iter"][j], n_evals=res["n_evals"][j],
                             truncated=res["truncated"][j])
+                        if inten is not None:
+                            dsets.update({k: v[j] for k, v in inten.items()})
                         dumper.append_attributes(**attrs)
                         dumper.append_datasets(**dsets)
                     if dumper is not None:

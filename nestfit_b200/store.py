@@ -50,6 +50,9 @@ HEADER_GROUPS = {'simple_header': 'simple_header', 'full_header': 'full_header'}
 RUN_ATTR_COLUMNS = ('null_lnZ', 'n_samples', 'n_live', 'global_lnZ', 'global_lnZ_err', 'max_loglike',
                     'BIC', 'AIC', 'AICc', 'null_BIC', 'null_AIC', 'null_AICc', 'n_iter', 'n_evals', 'truncated')
 RUN_DATASETS = ('posteriors', 'marginals', 'bestfit_params', 'map_params')
+# optional per-run datasets: posterior-weighted quantiles (M, n_spec, ncomp) of each component's peak (K) and
+# integrated (K km/s) intensity, written by fits run with intensity_marginals=True
+INTENSITY_DATASETS = ('peak_intensity_marginals', 'integrated_intensity_marginals')
 
 
 def run_attr_columns(ndim, n_chan_tot, nlive, null_lnZ, res, n_samples):
@@ -75,12 +78,19 @@ class Wave:
     """All runs of one ncomp of a pixel block, as they leave the sampler."""
 
     def __init__(self, ncomp, ndim, n_chan_tot, i_lon, i_lat, columns, row_offsets, posteriors, marginals,
-                 bestfit, mapfit):
+                 bestfit, mapfit, intensity=None):
+        """intensity: None, or {name: [n_run, M, n_spec, ncomp]} for the names of INTENSITY_DATASETS."""
         self.ncomp, self.ndim, self.n_chan_tot = int(ncomp), int(ndim), int(n_chan_tot)
         self.i_lon, self.i_lat = np.asarray(i_lon, dtype=np.int64), np.asarray(i_lat, dtype=np.int64)
         self.columns = columns
         self.row_offsets = np.asarray(row_offsets, dtype=np.int64)
         self.posteriors, self.marginals, self.bestfit, self.mapfit = posteriors, marginals, bestfit, mapfit
+        self.intensity = intensity
+
+    def dataset_names(self):
+        """The datasets of every run of this wave."""
+        names = [n for n in RUN_DATASETS if n != 'posteriors' or self.posteriors is not None]
+        return names + (list(INTENSITY_DATASETS) if self.intensity is not None else [])
 
     @property
     def n_run(self):
@@ -98,6 +108,8 @@ class Wave:
             return None if self.posteriors is None else self.posteriors[self.row_offsets[r]:self.row_offsets[r + 1]]
         if name == 'marginals':
             return self.marginals[r]
+        if name in INTENSITY_DATASETS:
+            return self.intensity[name][r]
         return (self.bestfit if name == 'bestfit_params' else self.mapfit)[r]
 
 
@@ -311,6 +323,9 @@ class GroupSink:
                 if name == 'posteriors' and not (self.store_posteriors and wave.posteriors is not None):
                     continue
                 sub.create_dataset(name, data=wave.run_dataset(r, name))
+            if wave.intensity is not None:
+                for name in INTENSITY_DATASETS:
+                    sub.create_dataset(name, data=wave.run_dataset(r, name))
 
     def add_pixels(self, i_lon, i_lat, nbest):
         for lon, lat, nb in zip(i_lon, i_lat, nbest):
@@ -363,7 +378,8 @@ class SlabSink:
             np.save(f'{stem}.post.npy', wave.posteriors)
         np.savez(f'{stem}.npz', ncomp=wave.ncomp, ndim=wave.ndim, n_chan_tot=wave.n_chan_tot, i_lon=wave.i_lon,
                  i_lat=wave.i_lat, row_offsets=wave.row_offsets, have_post=have_post, marginals=wave.marginals,
-                 bestfit=wave.bestfit, mapfit=wave.mapfit, **{f'col_{k}': v for k, v in wave.columns.items()})
+                 bestfit=wave.bestfit, mapfit=wave.mapfit, **{f'col_{k}': v for k, v in wave.columns.items()},
+                 **(wave.intensity if wave.intensity is not None else {}))
 
     def add_pixels(self, i_lon, i_lat, nbest):
         with self._lock:
@@ -386,9 +402,10 @@ class _SlabWave(Wave):
             post = None
             if bool(z['have_post']):
                 post = np.load(str(npz_path)[:-4] + '.post.npy', mmap_mode='r')
+            inten = {n: z[n] for n in INTENSITY_DATASETS} if INTENSITY_DATASETS[0] in z.files else None
             super().__init__(int(z['ncomp']), int(z['ndim']), int(z['n_chan_tot']), z['i_lon'], z['i_lat'],
                              {k: cols[k] for k in RUN_ATTR_COLUMNS}, z['row_offsets'], post, z['marginals'],
-                             z['bestfit'], z['mapfit'])
+                             z['bestfit'], z['mapfit'], inten)
 
 
 def read_slab_chunk(chunk_dir):
@@ -425,7 +442,7 @@ def slab_pix_tree(chunk_dirs, parent=None):
     def make_run(lon, lat, node, ncomp_key):
         wi, r = runs[lon][lat][int(ncomp_key)]
         wave = waves[wi]
-        names = [n for n in RUN_DATASETS if n != 'posteriors' or wave.posteriors is not None]
+        names = wave.dataset_names()
         return LazyGroup(f'/pix/{lon}/{lat}/{ncomp_key}', node, names, lambda n: np.asarray(wave.run_dataset(r, n)),
                          attrs=wave.run_attrs(r))
 
